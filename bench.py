@@ -243,6 +243,26 @@ def reference_cuda_rate(sd, B, iters=5):
 
 
 # ------------------------------------------------------------------------------------------------ this repo
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, **arrays):
+    """Writes each tensor as out_dir/<name>.npy in float32, so that two builds run with the same arguments (same seeded
+    inputs and weights) can be compared element for element.  When the tensors exceed DUMP_LIMIT_BYTES in all, each is
+    stored as every stride-th element of its flattened values, the same positions in every run.  Returns what was
+    written, for the JSON line."""
+    import numpy as np
+    total = sum(t.numel() for t in arrays.values()) * 4
+    stride = -(-total // DUMP_LIMIT_BYTES)
+    os.makedirs(out_dir, exist_ok=True)
+    written = {}
+    for name, t in arrays.items():
+        a = t.detach().float().flatten()[::stride].cpu().numpy() if stride > 1 else t.detach().float().cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+        written[name] = {"shape": list(t.shape), "stride": stride, "stored_elements": int(a.size)}
+    return {"dir": os.path.abspath(out_dir), "arrays": written}
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -277,15 +297,18 @@ def run_ours(args):
     sampler = ClockSampler(local) if rank == 0 else None
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     c_before = ops.LAUNCHES[0]
-    e0.record()
-    for _ in range(args.steps):
-        flush.zero_()
-        y = eng.forward(x_dev)
-    e1.record()
-    barrier()
+    try:
+        e0.record()
+        for _ in range(args.steps):
+            flush.zero_()
+            y = eng.forward(x_dev)
+        e1.record()
+        barrier()
+    finally:
+        clocks = sampler.stop() if sampler else None
     launches = ops.LAUNCHES[0] - c_before
     ms_step = max_over_ranks(e0.elapsed_time(e1), world) / args.steps
-    clocks = sampler.stop() if sampler else None
+    dumped = dump_outputs(args.dump_outputs, hr_frames=y) if args.dump_outputs and rank == 0 else None
 
     # ---------------- end-to-end through the public module API with host buffers (e2e)
     # Every step's clips start in pinned host memory and every step's HR frames end there, all inside the timed region.  The
@@ -335,7 +358,7 @@ def run_ours(args):
     e2e_u8 = None
     try:
         from edvr_b200 import frames_to_tensor, tensor_to_bytes
-        n8 = max(10, args.steps // 4)
+        n8 = args.steps
         f_host = torch.randint(0, 256, (B * 7, LR_H, LR_W, 3), dtype=torch.uint8).pin_memory()
         b_host = [torch.empty(B, 4 * LR_H, 4 * LR_W, 3, dtype=torch.uint8).pin_memory() for _ in range(2)]
         f_in = [torch.empty(B * 7, LR_H, LR_W, 3, dtype=torch.uint8, device="cuda") for _ in range(2)]
@@ -386,7 +409,7 @@ def run_ours(args):
         for _ in range(3):
             run1()
         barrier()
-        n1 = max(10, args.steps // 4)
+        n1 = args.steps
         e0.record()
         for _ in range(n1):
             flush.zero_()
@@ -440,6 +463,8 @@ def run_ours(args):
                                                  frac_hbm=prof["dcn"]["gbs"] / peak_hbm),
             "kernel_shares": prof["shares"],
         }
+        if dumped is not None:
+            line["dump_outputs"] = dumped
         if os.environ.get("EDVR_BENCH_PROFILING") == "1":
             # launch-list runs under ncu (profiles/): the baseline arms would only add minutes of serialised replays
             line["cpu_baseline"] = {"skipped": "EDVR_BENCH_PROFILING=1"}
@@ -499,20 +524,29 @@ def profile_step(eng, x):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200, help="timed steps (200 x ~25 ms: a 5 s timed region)")
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps of every timed loop (default 200 x ~25 ms: a 5 s timed region; 20 with --mode train, "
+                         "a training step being ~10x an inference step)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--mode", default="infer", choices=["infer", "train"])
     ap.add_argument("--clips", type=int, default=4, help="clips per GPU per step (8 runs into the 1 kW power cap)")
     ap.add_argument("--offset-std", type=float, default=0.02,
                     help="std of the random conv_offset init (0.02: ~0.02 px offsets; 3: several pixels)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the HR frames of the last timed step as DIR/hr_frames.npy (float32, at most 64 MB; "
+                         "inference with --impl ours)")
     args = ap.parse_args()
+    if args.steps is None:
+        args.steps = 20 if args.mode == "train" else 200
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.mode != "infer"):
+        ap.error("--dump-outputs is supported for inference with --impl ours")
     if args.impl == "reference":
         run_reference_arm(args)
     elif args.mode == "train":
         from edvr_b200 import train_bench
-        if args.steps == 200:
-            args.steps = 20          # a training step is ~10x an inference step; keep the default run within a minute
         train_bench.main(args)
     else:
         run_ours(args)

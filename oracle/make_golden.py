@@ -13,6 +13,9 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 OUT = os.path.join(os.path.dirname(HERE), "tests", "golden")
+# intra-op threads of every CPU graph recording: the CPU convolutions split their reductions by thread count, so a
+# bit-exact comparison with a recording runs with the same count (tests/test_oracle.py)
+RECORDING_THREADS = 8
 
 
 def reference_edvr(kwargs, seed):
@@ -50,6 +53,7 @@ CASES = {
 
 
 def main():
+    torch.set_num_threads(RECORDING_THREADS)
     os.makedirs(OUT, exist_ok=True)
     for name, (kw, shape) in CASES.items():
         net, _ = reference_edvr(kw, seed=11)

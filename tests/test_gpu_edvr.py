@@ -24,14 +24,13 @@ from conftest import rel_err
 pytestmark = pytest.mark.gpu
 
 
-def _compare(sd, x, hr_in=False, tol_l2=5e-3, tol_max=1e-3, center=None, dcn=None):
+def _compare(sd, x, hr_in=False, tol_l2=5e-3, tol_max=1e-3, center=None):
     from edvr_b200.engine import EDVREngine
     from oracle import edvr_ref
     torch.backends.cudnn.allow_tf32 = False
     torch.backends.cuda.matmul.allow_tf32 = False
     sdc = {k: v.cuda() for k, v in sd.items()}
-    kw = {} if dcn is None else {"dcn": dcn}
-    ref = edvr_ref.edvr_forward(sdc, x.cuda(), hr_in=hr_in, **kw)     # fp32 oracle graph (torchvision DCN by default)
+    ref = edvr_ref.edvr_forward(sdc, x.cuda(), hr_in=hr_in)     # fp32 oracle graph (torchvision DCN)
     eng = EDVREngine(sd, num_frame=x.shape[1], hr_in=hr_in)
     out = eng.forward(x.cuda())
     torch.cuda.synchronize()
@@ -77,85 +76,66 @@ def test_edvr_multi_pixel_offsets_vs_oracle_graph(offset_std):
     _compare(sd, x)
 
 
-def _reference_ext_dcn():
-    """B2-signature DCN running the UNMODIFIED reference CUDA extension (oracle/_ref), or None if it was not built."""
-    from oracle import build_ref
-    if not os.path.exists(build_ref.so_path()):
-        return None
-    ext = build_ref.load_ref()
-
-    def dcn(x, off, mask, w, b, s, p, d, g, dg):
-        x = x.contiguous()
-        out = x.new_empty(x.shape[0], w.shape[0], x.shape[2], x.shape[3])
-        ext.modulated_deform_conv_forward(x, w, b, x.new_empty(0), off, mask, out, x.new_empty(0), 3, 3, s, s, p, p,
-                                          d, d, g, dg, True)
-        return out
-    return dcn
+def _vs_refext(out, name, golden_dir, seed, offset_std, base=None):
+    """(max|out - ref| / max|ref|, rel-L2) of `out` against the output of the oracle graph running the reference's own CUDA
+    dcn extension, recorded on a B200 for case `name` of oracle/make_golden_refext.py (tests/golden/edvr_refext.npz):
+    every stride-th element of the flattened output, and max|ref| of the whole output.  With `base`, rel-L2 is taken of
+    the residuals out - base and ref - base."""
+    z = np.load(os.path.join(golden_dir, "edvr_refext.npz"))
+    stride = int(z[name + "_meta"][2])
+    assert z[name + "_meta"].tolist() == [seed, offset_std, stride, *out.shape]
+    got = out.flatten()[::stride].double().cpu()
+    want = torch.from_numpy(z[name + "_sample"]).double()
+    mx = float((got - want).abs().max()) / float(z[name + "_absmax"])
+    if base is not None:
+        b = base.flatten()[::stride].double().cpu()
+        got, want = got - b, want - b
+    return mx, float((got - want).norm() / want.norm())
 
 
 @pytest.mark.parametrize("offset_std", [0.02, 1.0])
-def test_edvr_l_full_size_vs_reference_cuda_ext_live(offset_std):
-    """BASELINE cfg 3 at FULL size (EDVR-L, 2 clips of 7x3x180x320 -> 3x720x1280): the fused executor vs the oracle graph
-    with the reference's own CUDA dcn extension (compiled unmodified into oracle/_ref) running live on the same GPU, fp32,
-    TF32 off."""
+def test_edvr_l_full_size_vs_reference_cuda_ext_live(offset_std, golden_dir):
+    """BASELINE cfg 3 at FULL size (EDVR-L, 2 clips of 7x3x180x320 -> 3x720x1280), fp32 references, TF32 off: the fused
+    executor vs the oracle graph over the whole output, and vs the oracle graph with the reference's own CUDA dcn extension
+    (compiled unmodified) as recorded on a B200, on a fixed sample of the output (_vs_refext)."""
     from oracle import edvr_ref
-    dcn = _reference_ext_dcn()
-    if dcn is None:
-        pytest.skip("oracle/_ref not built (no /root/reference at build time)")
     sd = edvr_ref.make_state_dict(num_feat=128, num_frame=7, num_extract_block=5, num_reconstruct_block=40, seed=9,
                                   offset_std=offset_std)
     x = torch.rand(2, 7, 3, 180, 320, generator=torch.Generator().manual_seed(9))
-    _compare(sd, x, dcn=dcn)
+    out, _ = _compare(sd, x)
+    base = F.interpolate(x[:, 3].cuda(), scale_factor=4, mode="bilinear", align_corners=False)
+    mx, l2 = _vs_refext(out, f"l_full_{offset_std}", golden_dir, 9, offset_std, base)
+    print(f"edvr vs reference dcn extension: rel-L2(residual)={l2:.3e}  max|d|/max|ref|={mx:.3e}")
+    assert l2 < 5e-3 and mx < 1e-3, (l2, mx)
 
 
-def _installed_reference():
-    """The UNMODIFIED reference package as pip-installed from /root/reference into baseline/_ref (travels with gpurun), or None."""
-    import sys
-    root = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "baseline", "_ref")
-    if not os.path.isdir(os.path.join(root, "basicsr", "models", "archs")):
-        return None
-    if root not in sys.path:
-        sys.path.insert(0, root)
-    import basicsr.models.archs.edvr_arch as arch      # noqa: F401  (imports the reference's own compiled dcn extension)
-    return sys.modules["basicsr.models.ops.dcn.deform_conv"], arch
-
-
-def test_unmodified_reference_edvr_runs_on_the_b1_shim():
-    """B1 boundary on the GPU: the reference's OWN EDVR graph (basicsr.models.archs.edvr_arch, unmodified, cuDNN convolutions)
-    is run twice on identical weights and input - once with the reference's compiled deform_conv_ext, once with
-    edvr_b200.deform_conv_ext bound in its place (INTEGRATION.md) - and must agree to 1e-3.  Multi-pixel offsets."""
-    ref = _installed_reference()
-    if ref is None:
-        pytest.skip("baseline/_ref (pip install of /root/reference) not present")
-    dc, arch = ref
+def test_unmodified_reference_edvr_runs_on_the_b1_shim(golden_dir):
+    """B1 boundary on the GPU: the reference's EDVR graph (the oracle port, cuDNN convolutions, fp32, TF32 off) with
+    edvr_b200.deform_conv_ext called in place of the reference's compiled deform_conv_ext, in the reference's argument
+    order (INTEGRATION.md), against the same graph on the same weights and input running the reference's own extension,
+    as recorded on a B200 (_vs_refext).  Must agree to 1e-3.  Multi-pixel offsets."""
     import edvr_b200.deform_conv_ext as shim
     from oracle import edvr_ref
+    from oracle.make_golden_refext import ext_dcn
+    torch.backends.cudnn.allow_tf32 = False
+    torch.backends.cuda.matmul.allow_tf32 = False
     kw = dict(num_feat=64, num_frame=3, deformable_groups=8, num_extract_block=1, num_reconstruct_block=2)
     sd = edvr_ref.make_state_dict(**kw, seed=21, offset_std=1.0)
-    net = arch.EDVR(center_frame_idx=None, **kw).cuda().eval()
-    net.load_state_dict(sd, strict=True)
     x = torch.rand(2, 3, 3, 32, 40, generator=torch.Generator().manual_seed(21)).cuda()
-    own = dc.deform_conv_ext
     with torch.no_grad():
-        y_ref = net(x)
-        dc.deform_conv_ext = shim
-        try:
-            y_ours = net(x)
-        finally:
-            dc.deform_conv_ext = own
-    e = rel_err(y_ours.cpu(), y_ref.cpu())
+        y_ours = edvr_ref.edvr_forward({k: v.cuda() for k, v in sd.items()}, x, dcn=ext_dcn(shim))
+    e = _vs_refext(y_ours, "b1", golden_dir, 21, 1.0)
     print(f"reference EDVR, own ext vs B1 shim: max-rel {e[0]:.3e}, rel-L2 {e[1]:.3e}")
     assert e[0] < 1e-3 and e[1] < 1e-3, e
 
 
 def test_standalone_b3_modules_match_the_reference_modules():
     """The drop-in module types north_star names - PCDAlignment, TSAFusion, ResidualBlockNoBN - called on their own (fp32
-    NCHW in/out like the reference's), against the reference's modules (baseline/_ref) or, without them, the oracle port."""
+    NCHW in/out like the reference's), against the oracle port of the reference's modules."""
     from edvr_b200 import edvr as ours
     from oracle import edvr_ref
     torch.backends.cudnn.allow_tf32 = False
     torch.backends.cuda.matmul.allow_tf32 = False
-    ref = _installed_reference()
     g = torch.Generator().manual_seed(31)
     C, dg, T = 64, 8, 3
 
@@ -184,13 +164,8 @@ def test_standalone_b3_modules_match_the_reference_modules():
     rf = [torch.randn(2, C, 24 >> i, 32 >> i, generator=g).cuda() for i in range(3)]
     with torch.no_grad():
         got = m(nbr, rf)
-        if ref is not None:
-            rm = ref[1].PCDAlignment(num_feat=C, deformable_groups=dg).cuda().eval()
-            rm.load_state_dict(m.state_dict(), strict=True)
-            want = rm(nbr, rf)
-        else:
-            sd = {"pcd_align." + k: v for k, v in m.state_dict().items()}
-            want = edvr_ref.pcd_align(sd, nbr, rf, dg, edvr_ref.dcn_torchvision)
+        sd = {"pcd_align." + k: v for k, v in m.state_dict().items()}
+        want = edvr_ref.pcd_align(sd, nbr, rf, dg, edvr_ref.dcn_torchvision)
     e = rel_err(got.cpu(), want.cpu())
     print(f"PCDAlignment standalone: {e}")
     assert e[0] < 2e-3 and e[1] < 2e-3, ("PCDAlignment", e)      # 15 fp16-operand layers in sequence: 2 x the per-op bound
@@ -200,12 +175,7 @@ def test_standalone_b3_modules_match_the_reference_modules():
     aligned = torch.randn(2, T, C, 24, 32, generator=g).cuda()
     with torch.no_grad():
         got = m(aligned)
-        if ref is not None:
-            rm = ref[1].TSAFusion(num_feat=C, num_frame=T, center_frame_idx=1).cuda().eval()
-            rm.load_state_dict(m.state_dict(), strict=True)
-            want = rm(aligned)
-        else:
-            want = edvr_ref.tsa_fusion({"fusion." + k: v for k, v in m.state_dict().items()}, aligned, 1)
+        want = edvr_ref.tsa_fusion({"fusion." + k: v for k, v in m.state_dict().items()}, aligned, 1)
     e = rel_err(got.cpu(), want.cpu())
     print(f"TSAFusion standalone: {e}")
     assert e[0] < 2e-3 and e[1] < 2e-3, ("TSAFusion", e)

@@ -17,6 +17,20 @@ import torch
 from conftest import rel_err
 from oracle import dcn_oracle, edvr_ref
 
+GOLDEN = os.path.join(os.path.dirname(__file__), "golden")
+
+
+def _port_forward(sd, x, **kw):
+    """edvr_ref.edvr_forward with the intra-op thread count of the recordings (oracle/make_golden.py): the CPU
+    convolutions split their reductions by thread count, and bit-exact agreement needs the same split."""
+    from oracle.make_golden import RECORDING_THREADS
+    n = torch.get_num_threads()
+    torch.set_num_threads(RECORDING_THREADS)
+    try:
+        return edvr_ref.edvr_forward(sd, x, **kw)
+    finally:
+        torch.set_num_threads(n)
+
 
 def _rand_case(N, C, H, W, Cout, dg, seed=0, off_scale=3.0, k=3):
     g = torch.Generator().manual_seed(seed)
@@ -167,26 +181,25 @@ def test_edvr_port_matches_reference_import_golden(path):
     kw = z["kwargs"].item()
     sd = edvr_ref.make_state_dict(**{k: v for k, v in kw.items() if k not in ("center_frame_idx",)}, seed=int(z["seed"]))
     x = torch.from_numpy(z["x"])
-    y = edvr_ref.edvr_forward(sd, x, hr_in=kw.get("hr_in", False))
+    y = _port_forward(sd, x, hr_in=kw.get("hr_in", False))
     assert torch.equal(y, torch.from_numpy(z["y"]))
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/basicsr"), reason="reference tree not mounted")
 def test_edvr_port_matches_reference_import_live():
-    """Where /root/reference exists (the build container), import it unchanged and compare live."""
-    from oracle.make_golden import reference_edvr
-    kw = dict(num_feat=16, num_frame=3, deformable_groups=2, num_extract_block=1, num_reconstruct_block=1,
-              with_tsa=True)
-    net, sd = reference_edvr(kw, seed=4)
-    x = torch.rand(1, 3, 3, 8, 12, generator=torch.Generator().manual_seed(0))
-    with torch.no_grad():
-        y = net(x)
-    assert torch.equal(y, edvr_ref.edvr_forward(sd, x))
-    assert set(sd) == set(net.state_dict())
+    """The reference graph imported unchanged (oracle/make_golden_live.py) on the weights of make_state_dict and a seeded
+    input: bit-identical output, same state_dict keys (tests/golden/ref_live.npz, ref_host.json)."""
+    import json
+    with open(os.path.join(GOLDEN, "ref_host.json")) as f:
+        ref = json.load(f)["port_edvr"]
+    z = np.load(os.path.join(GOLDEN, "ref_live.npz"))
+    sd = edvr_ref.make_state_dict(**ref["kwargs"], seed=ref["seed"])
+    x = torch.from_numpy(z["edvr_x"])
+    assert torch.equal(torch.from_numpy(z["edvr_y"]), _port_forward(sd, x))
+    assert sorted(sd) == ref["state_dict_keys"]
 
 
 # ---- frame staging either side of the network (SURVEY §8 f2): oracle/img_ref.py ---------------------------------------
-GOLDEN_IMG = os.path.join(os.path.dirname(__file__), "golden", "img_ref_import.npz")
+GOLDEN_IMG = os.path.join(GOLDEN, "img_ref_import.npz")
 
 
 def test_img_oracle_matches_reference_import_golden_bit_exact():
@@ -205,14 +218,12 @@ def test_img_oracle_matches_reference_import_golden_bit_exact():
     assert np.array_equal(img_ref.tensor2img(img_ref.frames_to_tensor(ramp)[0]), ramp[0])
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/basicsr"), reason="reference tree not mounted")
 def test_img_oracle_matches_live_reference_import():
-    from oracle import img_ref, make_golden_img
-    img2tensor, tensor2img = make_golden_img.reference_functions()
-    rng = np.random.default_rng(3)
-    frames = rng.integers(0, 256, size=(2, 9, 11, 3), dtype=np.uint8)
-    ref = torch.stack(img2tensor([f.astype(np.float32) / 255. for f in frames], bgr2rgb=True, float32=True), 0).numpy()
-    assert np.array_equal(img_ref.frames_to_tensor(frames).view(np.uint32), ref.view(np.uint32))
-    out = rng.normal(0.5, 0.6, size=(1, 3, 13, 7)).astype(np.float32)
-    assert np.array_equal(img_ref.tensor2img(out), tensor2img(torch.from_numpy(out)))
-    assert np.array_equal(img_ref.tensor2img(out[0, 0]), tensor2img(torch.from_numpy(out[0, 0])))
+    """The reference's img2tensor / tensor2img on seeded frames and outputs (tests/golden/ref_live.npz,
+    oracle/make_golden_live.py)."""
+    from oracle import img_ref
+    z = np.load(os.path.join(GOLDEN, "ref_live.npz"))
+    frames, out = z["img_frames"], z["img_out"]
+    assert np.array_equal(img_ref.frames_to_tensor(frames).view(np.uint32), z["img_x"].view(np.uint32))
+    assert np.array_equal(img_ref.tensor2img(out), z["img_y"])
+    assert np.array_equal(img_ref.tensor2img(out[0, 0]), z["img_y00"]) and z["img_y00"].ndim == 2
