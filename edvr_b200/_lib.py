@@ -11,7 +11,7 @@ LIB_PATH = os.environ.get("EDVR_B200_LIB", os.path.join(_HERE, "libedvr_b200.so"
 if os.environ.get("EDVR_B200_LIB"):      # development builds (e.g. the -DDP_PROF timing build of tools/dp_prof.py)
     LIB_PATH = os.environ["EDVR_B200_LIB"]
 
-ACT_NONE, ACT_RELU, ACT_LRELU, ACT_DCN_PACK, ACT_SIGMOID = 0, 1, 2, 3, 4
+ACT_NONE, ACT_RELU, ACT_LRELU, ACT_SIGMOID = 0, 1, 2, 4
 OUT_SAME, OUT_PIXSHUF2, OUT_STRIDE2 = 0, 1, 2
 
 c_int, c_void_p, c_float, c_size_t, c_ll = (ctypes.c_int, ctypes.c_void_p, ctypes.c_float,
@@ -29,7 +29,7 @@ class Epilogue(ctypes.Structure):
                 ("out16", c_void_p), ("out16_pix_stride", c_int), ("out16_ch_off", c_int),
                 ("out32", c_void_p), ("out32_pix_stride", c_int), ("out32_ch_off", c_int),
                 ("out_nchw", c_void_p), ("nchw_C", c_int), ("out_mode", c_int),
-                ("absmean_acc", c_void_p), ("f32_blocked", c_int), ("bf16", c_int)]
+                ("f32_blocked", c_int), ("bf16", c_int)]
 
 
 _SIGS = {
@@ -37,22 +37,20 @@ _SIGS = {
     "eb_last_error": (ctypes.c_char_p, []),
     "eb_selftest_umma": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
     "eb_packed_weight_bytes": (c_size_t, [c_int] * 4),
-    "eb_pack_weight": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p]),
+    "eb_pack_weight": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),
     "eb_conv2d": (c_int, [ctypes.POINTER(Src), c_int, c_int, c_int, c_int, c_int, c_void_p, c_int, c_int,
                           ctypes.POINTER(Epilogue), c_void_p]),
     "eb_conv2d_stats": (c_int, [ctypes.POINTER(Src), c_int, c_int, c_int, c_int, c_int, c_void_p, c_int, c_int,
                                 ctypes.POINTER(Epilogue), c_void_p, c_void_p]),
     "eb_conv2d_pair_supported": (c_int, [c_int] * 4),
-    "eb_pack_weight_pair": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_int, c_void_p, c_void_p]),
-    "eb_pack_weight_pair_ex": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_int, c_void_p, c_int, c_void_p]),
+    "eb_pack_weight_pair": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),
+    "eb_pack_weight_pair_ex": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_int, c_void_p]),
     "eb_pack_weight_pair_dgrad": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_int, c_void_p]),
     "eb_conv_wgrad_workspace": (c_size_t, [c_int] * 6),
     "eb_conv_wgrad": (c_int, [c_void_p, c_int, c_int, c_void_p, c_int, c_int] + [c_int] * 7 + [c_float, c_void_p, c_void_p, c_void_p,
                                                                                            c_size_t, c_void_p]),
     "eb_conv2d_pair": (c_int, [ctypes.POINTER(Src), c_int, c_int, c_int, c_int, c_int, c_void_p, c_int, c_int,
                                ctypes.POINTER(Epilogue), c_void_p]),
-    "eb_dcn_nhwc": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_int,
-                            c_void_p, c_int, c_int, ctypes.POINTER(Epilogue), c_void_p]),
     "eb_dcn_site_offset_weight_bytes": (c_size_t, [c_int]),
     "eb_dcn_site_pack_offset_weight": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p]),
     "eb_dcn_site": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int,

@@ -83,7 +83,6 @@ int fill_epi(const eb_epilogue_t* e, int H, int W, int cout_packed, EpiParams* o
     o->out_nchw = e->out_nchw;
     o->nchw_C = e->nchw_C;
     o->out_mode = e->out_mode;
-    o->absmean_acc = e->absmean_acc;
     o->f32_blocked = e->f32_blocked;
     o->bf16 = e->bf16;
     o->res16_wide = (e->res16 && reinterpret_cast<uintptr_t>(e->res16) % 32 == 0 && e->res_pix_stride % 16 == 0 &&
@@ -91,7 +90,7 @@ int fill_epi(const eb_epilogue_t* e, int H, int W, int cout_packed, EpiParams* o
     if (e->f32_blocked && (e->out_mode != EB_OUT_SAME || (e->out32 && (e->out32_pix_stride % 32 || e->out32_ch_off % 32)) ||
                            (e->res32 && (e->res_pix_stride % 32 || e->res_ch_off % 32)) || e->res16))
         return fail(EB_ERR_UNSUPPORTED, "f32_blocked needs OUT_SAME, C %% 32 == 0, and no fp16 residual");
-    if (e->act < EB_ACT_NONE || e->act > EB_ACT_SIGMOID) return fail(EB_ERR_UNSUPPORTED, "act %d", e->act);
+    if (e->act < EB_ACT_NONE || e->act > EB_ACT_SIGMOID || e->act == 3) return fail(EB_ERR_UNSUPPORTED, "act %d", e->act);
     if (e->out_mode < EB_OUT_SAME || e->out_mode > EB_OUT_STRIDE2)
         return fail(EB_ERR_UNSUPPORTED, "out_mode %d", e->out_mode);
     if (!e->out16 && !e->out32 && !e->out_nchw) return fail(EB_ERR_NULLPTR, "no output pointer");
@@ -120,7 +119,7 @@ int set_smem(KernelT k, int bytes) {
 
 extern "C" {
 
-int eb_version(void) { return 100; }
+int eb_version(void) { return 101; }
 const char* eb_last_error(void) { return g_err; }
 
 int eb_selftest_umma(const void* A, const void* B, float* D, int N, int K, int variant, void* stream) {
@@ -166,15 +165,14 @@ size_t eb_packed_weight_bytes(int cin, int ktaps, int BN, int n_tiles_n) {
     return static_cast<size_t>(n_tiles_n) * BN * cin * ktaps * 2;
 }
 
-int eb_pack_weight(const float* w, int cout, int cin, int ktaps, const int* row_map, int BN,
-                   int n_tiles_n, int tap_major, void* wpack, void* stream) {
+int eb_pack_weight(const float* w, int cout, int cin, int ktaps, int BN, int n_tiles_n, void* wpack, void* stream) {
     if (!w || !wpack) return fail(EB_ERR_NULLPTR, "pack_weight: null pointer");
     if (cin % 64 || BN % 32 || BN < 32 || BN > 128 || n_tiles_n < 1 || ktaps < 1 || cout < 1)
         return fail(EB_ERR_INVALID_SHAPE, "pack_weight: cin=%d BN=%d tiles=%d taps=%d", cin, BN, n_tiles_n, ktaps);
-    if (!row_map && cout > BN * n_tiles_n) return fail(EB_ERR_INVALID_SHAPE, "pack_weight: cout exceeds packed rows");
+    if (cout > BN * n_tiles_n) return fail(EB_ERR_INVALID_SHAPE, "pack_weight: cout exceeds packed rows");
     const long long groups = static_cast<long long>(n_tiles_n) * (cin / 64) * ktaps * 8 * BN;
     pack_weight_kernel<<<grid_1d(groups, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
-        w, cout, cin, ktaps, row_map, BN, n_tiles_n, tap_major, static_cast<__half*>(wpack));
+        w, cout, cin, ktaps, BN, n_tiles_n, static_cast<__half*>(wpack));
     return check_launch("pack_weight");
 }
 
@@ -212,24 +210,23 @@ static int encode_halo_map(const ConvSrc& S, int H, int W, int n_images, int tap
     return EB_OK;
 }
 
-int eb_pack_weight_pair(const float* w, int cout, int cin, int ktaps, const int* row_map, int BN, int n_tiles_n,
-                        void* wpack, void* stream) {
-    return eb_pack_weight_pair_ex(w, cout, cin, ktaps, row_map, BN, n_tiles_n, wpack, 0, stream);
+int eb_pack_weight_pair(const float* w, int cout, int cin, int ktaps, int BN, int n_tiles_n, void* wpack, void* stream) {
+    return eb_pack_weight_pair_ex(w, cout, cin, ktaps, BN, n_tiles_n, wpack, 0, stream);
 }
 
-int eb_pack_weight_pair_ex(const float* w, int cout, int cin, int ktaps, const int* row_map, int BN, int n_tiles_n,
-                           void* wpack, int bf16, void* stream) {
+int eb_pack_weight_pair_ex(const float* w, int cout, int cin, int ktaps, int BN, int n_tiles_n, void* wpack, int bf16,
+                           void* stream) {
     if (!w || !wpack) return fail(EB_ERR_NULLPTR, "pack_weight_pair: null pointer");
     if (cin % 64 || BN % 32 || BN < 32 || BN > 128 || n_tiles_n < 1 || ktaps < 1 || cout < 1)
         return fail(EB_ERR_INVALID_SHAPE, "pack_weight_pair: cin=%d BN=%d tiles=%d taps=%d", cin, BN, n_tiles_n, ktaps);
-    if (!row_map && cout > BN * n_tiles_n) return fail(EB_ERR_INVALID_SHAPE, "pack_weight_pair: cout exceeds packed rows");
+    if (cout > BN * n_tiles_n) return fail(EB_ERR_INVALID_SHAPE, "pack_weight_pair: cout exceeds packed rows");
     const long long groups = static_cast<long long>(n_tiles_n) * BN * (cin / 8) * ktaps;
     if (bf16)
         pack_weight_pair_kernel<true><<<grid_1d(groups, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
-            w, cout, cin, ktaps, row_map, BN, n_tiles_n, static_cast<__half*>(wpack));
+            w, cout, cin, ktaps, BN, n_tiles_n, static_cast<__half*>(wpack));
     else
         pack_weight_pair_kernel<false><<<grid_1d(groups, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
-            w, cout, cin, ktaps, row_map, BN, n_tiles_n, static_cast<__half*>(wpack));
+            w, cout, cin, ktaps, BN, n_tiles_n, static_cast<__half*>(wpack));
     return check_launch("pack_weight_pair");
 }
 
@@ -282,7 +279,6 @@ static int launch_conv(const ConvParams& P, cudaStream_t st) {
         const EpiParams& e = P.epi;
         if (e.out_mode == OUT_PIXSHUF2) ek = EK_PIXSHUF;
         else if (e.out_mode == OUT_STRIDE2) ek = EK_STRIDE2;
-        else if (e.act == ACT_DCN_PACK) { if (e.out16 && !e.out32 && !e.res16 && !e.res32) ek = EK_PACK; }
         else if (e.out32 || e.res32) { if (!e.res16) ek = EK_F32; }
         else if (e.out16) ek = EK_PLAIN;
     }
@@ -310,7 +306,6 @@ static int launch_conv(const ConvParams& P, cudaStream_t st) {
         switch (ek) {
             case EK_PLAIN: EB_DISPATCH_C2(EK_PLAIN); break;
             case EK_F32: EB_DISPATCH_C2(EK_F32); break;
-            case EK_PACK: EB_DISPATCH_C2(EK_PACK); break;
             case EK_PIXSHUF: EB_DISPATCH_C2(EK_PIXSHUF); break;
             default: EB_DISPATCH_C2(EK_STRIDE2); break;
         }
@@ -327,7 +322,6 @@ static int launch_conv(const ConvParams& P, cudaStream_t st) {
         const bool plain_out = e.out16 && !e.out32 && !e.res32 && !e.out_nchw;
         if (e.out_mode == OUT_PIXSHUF2) ek1 = EK_PIXSHUF;
         else if (e.out_mode == OUT_STRIDE2) ek1 = EK_STRIDE2;
-        else if (e.act == ACT_DCN_PACK) { if (plain_out && !e.res16) ek1 = EK_PACK; }
         else if (plain_out) ek1 = EK_PLAIN;
         else if ((e.out32 || e.res32) && !e.res16 && !e.out_nchw) ek1 = EK_F32;
     }
@@ -341,7 +335,6 @@ static int launch_conv(const ConvParams& P, cudaStream_t st) {
         switch (ek1) {                                                                                 \
             case EK_PLAIN: EB_LAUNCH_C1(HALO_, EK_PLAIN); break;                                       \
             case EK_F32: EB_LAUNCH_C1(HALO_, EK_F32); break;                                           \
-            case EK_PACK: EB_LAUNCH_C1(HALO_, EK_PACK); break;                                         \
             case EK_PIXSHUF: EB_LAUNCH_C1(HALO_, EK_PIXSHUF); break;                                   \
             case EK_STRIDE2: EB_LAUNCH_C1(HALO_, EK_STRIDE2); break;                                   \
             default: EB_LAUNCH_C1(HALO_, EK_GENERIC); break;                                           \
@@ -420,7 +413,6 @@ int eb_conv2d_pair(const eb_src_t* srcs, int nsrc, int N, int H, int W, int ksiz
         const bool plain_out = e.out16 && !e.out32 && !e.res32 && !e.out_nchw;
         if (e.out_mode == OUT_PIXSHUF2) ek1 = EK_PIXSHUF;
         else if (e.out_mode == OUT_STRIDE2) ek1 = EK_STRIDE2;
-        else if (e.act == ACT_DCN_PACK) { if (plain_out && !e.res16) ek1 = EK_PACK; }
         else if (plain_out) ek1 = EK_PLAIN;
         else if ((e.out32 || e.res32) && !e.res16 && !e.out_nchw) ek1 = EK_F32;
     }
@@ -447,10 +439,10 @@ int eb_conv2d_pair(const eb_src_t* srcs, int nsrc, int N, int H, int W, int ksiz
                                CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
         if (r != CUDA_SUCCESS) return fail(EB_ERR_LAUNCH, "conv2d_pair: weight tensor map failed (%d)", static_cast<int>(r));
     }
-    // fp16 NHWC output through TMA when the epilogue writes it pixel-for-pixel (plain / fp32-stream / DCN-record kinds)
+    // fp16 NHWC output through TMA when the epilogue writes it pixel-for-pixel (plain / fp32-stream kinds)
     PP.tma_out = 0;
     PP.tmap_out = PP.tmap[0];
-    if ((ek1 == EK_PLAIN || ek1 == EK_F32 || ek1 == EK_PACK) && P.epi.out16 != nullptr && !(P.dbg & 64)) {
+    if ((ek1 == EK_PLAIN || ek1 == EK_F32) && P.epi.out16 != nullptr && !(P.dbg & 64)) {
         eb_encode_tiled_fn enc = tensor_map_encoder();
         const cuuint64_t ps = static_cast<cuuint64_t>(P.epi.out16_pix_stride);
         const cuuint64_t dims[4] = {ps, static_cast<cuuint64_t>(W), static_cast<cuuint64_t>(H), static_cast<cuuint64_t>(N)};
@@ -507,7 +499,6 @@ int eb_conv2d_pair(const eb_src_t* srcs, int nsrc, int N, int H, int W, int ksiz
     switch (ek1) {
         case EK_PLAIN: if (PP.tma_out) EB_LAUNCH_CP(EK_PLAIN, true); else EB_LAUNCH_CP(EK_PLAIN, false); break;
         case EK_F32: if (PP.tma_out) EB_LAUNCH_CP(EK_F32, true); else EB_LAUNCH_CP(EK_F32, false); break;
-        case EK_PACK: if (PP.tma_out) EB_LAUNCH_CP(EK_PACK, true); else EB_LAUNCH_CP(EK_PACK, false); break;
         case EK_PIXSHUF: if (PP.tma_out) EB_LAUNCH_CP(EK_PIXSHUF, true); else EB_LAUNCH_CP(EK_PIXSHUF, false); break;
         case EK_STRIDE2: EB_LAUNCH_CP(EK_STRIDE2, false); break;
         default: EB_LAUNCH_CP(EK_GENERIC, false); break;
@@ -515,55 +506,6 @@ int eb_conv2d_pair(const eb_src_t* srcs, int nsrc, int N, int H, int W, int ksiz
 #undef EB_LAUNCH_CP
     if (err != cudaSuccess) return fail(EB_ERR_LAUNCH, "conv2d_pair: %s", cudaGetErrorString(err));
     return check_launch("conv_pair");
-}
-
-static int launch_dcn(DcnParams& P, cudaStream_t st) {
-    P.x_wide = (P.cpg % 16 == 0 && P.x_pix_stride % 16 == 0 && P.x_ch_off % 16 == 0 &&
-                reinterpret_cast<uintptr_t>(P.x) % 32 == 0 && getenv("EDVR_B200_DCN_NARROW") == nullptr) ? 1 : 0;
-    const long long tiles = static_cast<long long>(P.N) * ((P.Ho + DC_TILE_H - 1) / DC_TILE_H) *
-                            ((P.Wo + DC_TILE_W - 1) / DC_TILE_W) * P.n_tiles_n;
-    if (tiles == 0) return EB_OK;
-    const int grid = static_cast<int>(tiles < num_sms() ? tiles : num_sms());
-    // keep the rest of the 228 KB for L1: the nine taps of a chunk re-read the same slab of x
-    static const int carve = (DC_SMEM_BYTES + 1024) * 100 / (228 * 1024) + 1;
-    const bool nchw = P.epi.out_nchw != nullptr;
-    if (nchw && (P.epi.out16 || P.epi.out32 || P.epi.res16 || P.epi.res32)) return fail(EB_ERR_UNSUPPORTED, "dcn: NCHW output excludes other outputs");
-    if (!nchw && (!P.epi.out16 || P.epi.out32 || P.epi.res32 || P.epi.res16)) return fail(EB_ERR_UNSUPPORTED, "dcn: NHWC fp16 output only");
-#define EB_LAUNCH_DCN(OFF_, EK_)                                                                                     \
-    do {                                                                                                             \
-        cudaFuncSetAttribute(dcn_fused_kernel<OFF_, EK_>, cudaFuncAttributePreferredSharedMemoryCarveout, carve);    \
-        if (int rc = set_smem(dcn_fused_kernel<OFF_, EK_>, DC_SMEM_BYTES)) return rc;                                \
-        dcn_fused_kernel<OFF_, EK_><<<grid, DC_THREADS, DC_SMEM_BYTES, st>>>(P);                                     \
-    } while (0)
-    if (P.off_mode == OFF_NCHW_F32) { if (nchw) EB_LAUNCH_DCN(OFF_NCHW_F32, EK_NCHW); else EB_LAUNCH_DCN(OFF_NCHW_F32, EK_PLAIN); }
-    else                            { if (nchw) EB_LAUNCH_DCN(OFF_PACK_F16, EK_NCHW); else EB_LAUNCH_DCN(OFF_PACK_F16, EK_PLAIN); }
-#undef EB_LAUNCH_DCN
-    return check_launch("dcn_fused");
-}
-
-int eb_dcn_nhwc(const void* x, int x_pix_stride, int x_ch_off, int N, int H, int W, int C, int dg,
-                const void* offpack, int offpack_pix_stride, const void* wpack, int BN, int n_tiles_n,
-                const eb_epilogue_t* epi, void* stream) {
-    if (!x || !offpack || !wpack) return fail(EB_ERR_NULLPTR, "dcn_nhwc: null pointer");
-    if (N < 0 || H < 1 || W < 1 || C < 64 || C % 64 || dg < 1 || C % dg || (C / dg) % 8)
-        return fail(EB_ERR_INVALID_SHAPE, "dcn_nhwc: N=%d H=%d W=%d C=%d dg=%d", N, H, W, C, dg);
-    if (BN % 32 || BN < 32 || BN > 128 || n_tiles_n < 1 || BN * n_tiles_n > DC_MAX_COUT)
-        return fail(EB_ERR_INVALID_SHAPE, "dcn_nhwc: BN=%d n_tiles_n=%d", BN, n_tiles_n);
-    if (!al16(x) || !al16(offpack) || !al16(wpack) || x_pix_stride % 8 || x_ch_off % 8 ||
-        offpack_pix_stride % 8 || offpack_pix_stride < dg * 32)
-        return fail(EB_ERR_ALIGNMENT, "dcn_nhwc: views must be 16-byte aligned");
-    DcnParams P;
-    memset(&P, 0, sizeof(P));
-    P.x = static_cast<const __half*>(x); P.x_pix_stride = x_pix_stride; P.x_ch_off = x_ch_off;
-    P.N = N; P.H = H; P.W = W; P.C = C; P.Ho = H; P.Wo = W;
-    P.kh = 3; P.kw = 3; P.stride = 1; P.pad = 1; P.dil = 1; P.stride_w = 1; P.pad_w = 1; P.dil_w = 1;
-    P.dg = dg; P.cpg = C / dg;
-    P.off_mode = OFF_PACK_F16;
-    P.offpack = static_cast<const __half*>(offpack); P.offpack_pix_stride = offpack_pix_stride;
-    P.wpack = static_cast<const __half*>(wpack); P.BN = BN; P.n_tiles_n = n_tiles_n;
-    if (int rc = fill_epi(epi, H, W, BN * n_tiles_n, &P.epi)) return rc;
-    if (P.epi.out_mode != OUT_SAME) return fail(EB_ERR_UNSUPPORTED, "dcn_nhwc: out_mode");
-    return launch_dcn(P, static_cast<cudaStream_t>(stream));
 }
 
 // ---- training step: weight gradient of a dense 3x3 (pad 1) / 1x1 convolution (conv_train.cuh)
@@ -706,7 +648,7 @@ int eb_dcn_site(const void* x, int x_pix_stride, int x_ch_off, int N, int H, int
     P.kh = 3; P.kw = 3; P.stride = 1; P.pad = 1; P.dil = 1; P.stride_w = 1; P.pad_w = 1; P.dil_w = 1;
     P.dg = dg; P.cpg = C / dg;
     P.x_wide = (x_pix_stride % 16 == 0 && x_ch_off % 16 == 0 && reinterpret_cast<uintptr_t>(x) % 32 == 0) ? 1 : 0;
-    P.off_mode = OFF_NCHW_F32; P.offset = offset; P.mask = mask;
+    P.offset = offset; P.mask = mask;
     P.wpack = static_cast<const __half*>(wpack); P.BN = BN; P.n_tiles_n = n_tiles_n;
     if (int rc = fill_epi(epi, H, W, BN * n_tiles_n, &P.epi)) return rc;
     if (P.epi.out_mode != OUT_SAME) return fail(EB_ERR_UNSUPPORTED, "dcn_site: out_mode");
@@ -971,8 +913,8 @@ int dcn_forward_impl(const char* who, const float* x, const float* offset, const
         else nchw_f32_to_nhwc_f16_kernel<<<grid, block, 0, st>>>(x, x16, C, H * W, C, 0);
         if (int rc = check_launch("nchw_to_nhwc")) return rc;
     }
-    if (int rc = eb_pack_weight(weight, Cout, C, kh * kw, nullptr, BN, nt, 0, wpack, stream)) return rc;
-    pack_bias_kernel<<<(BN * nt + 127) / 128, 128, 0, st>>>(bias, Cout, nullptr, BN * nt, bpack);
+    if (int rc = eb_pack_weight(weight, Cout, C, kh * kw, BN, nt, wpack, stream)) return rc;
+    pack_bias_kernel<<<(BN * nt + 127) / 128, 128, 0, st>>>(bias, Cout, BN * nt, bpack);
     if (int rc = check_launch("pack_bias")) return rc;
 
     DcnParams P;
@@ -981,11 +923,19 @@ int dcn_forward_impl(const char* who, const float* x, const float* offset, const
     P.N = N; P.H = H; P.W = W; P.C = C; P.Ho = Ho; P.Wo = Wo;
     P.kh = kh; P.kw = kw; P.stride = g.sh; P.pad = g.ph; P.dil = g.dh; P.stride_w = g.sw; P.pad_w = g.pw; P.dil_w = g.dw;
     P.dg = dg; P.cpg = C / dg;
-    P.off_mode = OFF_NCHW_F32; P.offset = offset; P.mask = mask;
+    P.x_wide = (P.cpg % 16 == 0 && reinterpret_cast<uintptr_t>(x16) % 32 == 0) ? 1 : 0;   // pixel stride C % 64 == 0, offset 0
+    P.offset = offset; P.mask = mask;
     P.wpack = wpack; P.BN = BN; P.n_tiles_n = nt;
     P.epi.bias = bias ? bpack : nullptr; P.epi.act = ACT_NONE; P.epi.H = Ho; P.epi.W = Wo;
     P.epi.out_nchw = out; P.epi.nchw_C = Cout; P.epi.out_mode = OUT_SAME;
-    return launch_dcn(P, st);
+    const long long tiles = static_cast<long long>(N) * ((Ho + DC_TILE_H - 1) / DC_TILE_H) * ((Wo + DC_TILE_W - 1) / DC_TILE_W) * nt;
+    const int grid = static_cast<int>(tiles < num_sms() ? tiles : num_sms());
+    // keep the rest of the 228 KB for L1: the nine taps of a chunk re-read the same slab of x
+    static const int carve = (DC_SMEM_BYTES + 1024) * 100 / (228 * 1024) + 1;
+    cudaFuncSetAttribute(dcn_fused_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, carve);
+    if (int rc = set_smem(dcn_fused_kernel, DC_SMEM_BYTES)) return rc;
+    dcn_fused_kernel<<<grid, DC_THREADS, DC_SMEM_BYTES, st>>>(P);
+    return check_launch("dcn_fused");
 }
 }  // namespace
 

@@ -443,7 +443,7 @@ __device__ __forceinline__ float2 unpack_h2(uint32_t u) {
 __device__ __forceinline__ float sigmoidf_fast(float x) { return 1.0f / (1.0f + __expf(-x)); }
 
 // activation codes shared by host and device
-enum : int { ACT_NONE = 0, ACT_RELU = 1, ACT_LRELU = 2, ACT_DCN_PACK = 3, ACT_SIGMOID = 4 };
+enum : int { ACT_NONE = 0, ACT_RELU = 1, ACT_LRELU = 2, ACT_SIGMOID = 4 };
 
 __device__ __forceinline__ float apply_act(float v, int act) {
     if (act == ACT_RELU) return fmaxf(v, 0.0f);

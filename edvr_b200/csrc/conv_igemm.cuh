@@ -224,8 +224,6 @@ __global__ void __launch_bounds__(CV_THREADS, 1) conv_igemm_kernel(const ConvPar
         const int q = warp & 3;
         const int sub = (warp - 6) >> 2;
         uint32_t acc_it = 0;
-        float abs_sum = 0.f;
-        float* const abs_ptr = ((EK == EK_PACK || EK == EK_GENERIC) && P.epi.absmean_acc != nullptr) ? &abs_sum : nullptr;
         for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x, ++acc_it) {
             const int nt = tile % P.n_tiles_n, pt = tile / P.n_tiles_n;
             const int tx = pt % tiles_x, ty = (pt / tiles_x) % tiles_y, img = pt / (tiles_x * tiles_y);
@@ -240,13 +238,12 @@ __global__ void __launch_bounds__(CV_THREADS, 1) conv_igemm_kernel(const ConvPar
             for (int cc = 0; cc < ((P.dbg & 4) ? 0 : P.BN); cc += 32) {
                 float v[32];
                 tmem_ld32(t0 + cc, v);
-                epi_store32<EK>(P.epi, has_bias ? bias_s : nullptr, v, img, y, x, nt * P.BN + cc, valid, abs_ptr);
+                epi_store32<EK>(P.epi, has_bias ? bias_s : nullptr, v, img, y, x, nt * P.BN + cc, valid);
             }
             tc_fence_before_sync();
             __syncwarp();
             if (lane == 0) mbar_arrive(&acc_empty[ab]);
         }
-        if (abs_ptr != nullptr) epi_flush_abs_sum(P.epi, abs_sum);
     }
 
     // ---- teardown

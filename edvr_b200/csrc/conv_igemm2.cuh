@@ -206,7 +206,6 @@ __global__ void __launch_bounds__(C2_THREADS, 1) conv_igemm2_kernel(const ConvPa
         const int q = warp & 3;
         const EpiParams E = P.epi;
         const int H = P.H, W = P.W, NIMG = P.N, dbg = STATS ? P.dbg : 0;
-        const int act1 = (EK == EK_PACK) ? ACT_NONE : E.act;
         const long long ps16 = PS ? PS : E.out16_pix_stride, ps32 = PS ? PS : E.out32_pix_stride,
                         psr = PS ? PS : E.res_pix_stride;
         uint32_t acc_it = 0;
@@ -226,7 +225,7 @@ __global__ void __launch_bounds__(C2_THREADS, 1) conv_igemm2_kernel(const ConvPa
             const __half* r16 = nullptr;
             const float* r32 = nullptr;
             long long ops16 = ps16, orow16 = static_cast<long long>(W) * ps16;   // element strides of the fp16 output
-            if (EK == EK_PLAIN || EK == EK_F32 || EK == EK_PACK) {
+            if (EK == EK_PLAIN || EK == EK_F32) {
                 if (E.out16 != nullptr) o16 = E.out16 + E.out16_ch_off + co + pix0 * ps16;
                 if (EK == EK_F32 && E.out32 != nullptr) o32 = E.out32 + E.out32_ch_off + co + pix0 * ps32;
                 if (EK == EK_PLAIN && E.res16 != nullptr) r16 = E.res16 + E.res_ch_off + co + pix0 * psr;
@@ -255,27 +254,11 @@ __global__ void __launch_bounds__(C2_THREADS, 1) conv_igemm2_kernel(const ConvPa
                 if (STATS) { const long long t = clock64(); st_acc[ST_E_TMEM] += t - tq; tq = t; }
 #pragma unroll
                 for (int j = 0; j < 32; ++j) v[j] += bias_c;
-                act_inplace<32>(v, act1);
+                act_inplace<32>(v, E.act);
                 const int yb = col >> 3;                                   // first tile row of these 32 pixels
-                if (EK == EK_PACK) {
-                    // packed DCN record: channel j = co % 32 = lane: [0,18) offsets, [18,27) mask logits, rest pad
-                    float s = 0.f;
-                    if (lane >= 18 && lane < 27) {
-#pragma unroll
-                        for (int e = 0; e < 32; ++e) v[e] = sigmoidf_fast(v[e]);
-                    } else if (lane < 18 && E.absmean_acc != nullptr && img_ok) {
-#pragma unroll
-                        for (int e = 0; e < 32; ++e) s += ((y0 + yb + (e >> 3) < H) && ((e & 7) < xn)) ? fabsf(v[e]) : 0.f;
-                    }
-                    if (E.absmean_acc != nullptr) {
-#pragma unroll
-                        for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-                        if (lane == 0 && img_ok) atomicAdd(E.absmean_acc, s);
-                    }
-                }
                 if (STATS) { const long long t = clock64(); st_acc[ST_E_P1] += t - tq; tq = t; }
                 if (img_ok && !(dbg & 2)) {
-                    if (EK == EK_PLAIN || EK == EK_PACK) {
+                    if (EK == EK_PLAIN) {
                         if (interior) {
                             // full tile: straight-line code, no predicates (keeps the loop inside the L0 I-cache)
 #pragma unroll

@@ -253,8 +253,6 @@ __global__ void __launch_bounds__(CP_THREADS, 1) conv_pair_kernel(const __grid_c
             const uint32_t st_row = smem_u32(stage) + lane * 64;
             const uint32_t st_x = ((lane >> 1) & 3) * 16;
             uint32_t acc_it = 0;
-            float abs_sum = 0.f;
-            float* const abs_ptr = (EK == EK_PACK && P.epi.absmean_acc != nullptr) ? &abs_sum : nullptr;
             for (int t = ci; t < total_pt; t += cpn, ++acc_it) {
                 const int tx = (t % tiles_x2) * 2 + static_cast<int>(rank), ty = (t / tiles_x2) % tiles_y;
                 const int img = t / (tiles_x2 * tiles_y);
@@ -278,7 +276,7 @@ __global__ void __launch_bounds__(CP_THREADS, 1) conv_pair_kernel(const __grid_c
                 auto do_chunk = [&](int cc, const float4* pre) {
                     float v[32];
                     tmem_ld32(t0 + cc, v);
-                    epi_store32<EK, TMA_OUT>(P.epi, has_bias ? bias_s - nt * P.BN : nullptr, v, img, y, x, nt * P.BN + cc, valid, abs_ptr, pre);
+                    epi_store32<EK, TMA_OUT>(P.epi, has_bias ? bias_s - nt * P.BN : nullptr, v, img, y, x, nt * P.BN + cc, valid, pre);
                     if (TMA_OUT && EK == EK_PIXSHUF) {
                         // PixelShuffle(2): conv channel 4k + 2i + j of pixel (y, x) is output channel k of pixel (2y+i, 2x+j)
                         // (edvr_arch.py:351,410-411).  Staging = the 8 x 16 output pixels of this warp, 8 channels (16 B) each,
@@ -347,7 +345,6 @@ __global__ void __launch_bounds__(CP_THREADS, 1) conv_pair_kernel(const __grid_c
                 __syncwarp();
                 if (lane == 0) { if (leader) mbar_arrive(&acc_empty[ab]); else mbar_arrive_remote(&acc_empty[ab], 0); }
             }
-            if (abs_ptr != nullptr) epi_flush_abs_sum(P.epi, abs_sum);
             if (TMA_OUT && lane == 0) bulk_wait_group0();        // all output boxes written before the CTA retires
         }
     }

@@ -8,13 +8,13 @@
 // input (16 B = 8 channels per corner load), apply the modulation mask and write the result
 // straight into the shared-memory A operand (no-swizzle K-major planes, common.cuh); one
 // thread issues tcgen05.mma against the pre-packed weights (B operand, bulk async copies);
-// the fp32 accumulator lives in TMEM and is drained by four epilogue warps (bias, activation,
-// NHWC fp16 and/or NCHW fp32 stores).  K is walked chunk-major: stage = (64-channel chunk, tap), so the nine
+// the fp32 accumulator lives in TMEM and is drained by four epilogue warps (bias, NCHW fp32
+// store).  Offsets and masks arrive fp32 NCHW in the reference layout.  K is walked chunk-major: stage = (64-channel chunk, tap), so the nine
 // taps of a chunk re-read the same ~23 KB slab of x and hit L1.
 // Gather mapping (L1TEX wavefronts and issue slots are the limiters of this kernel, profiles/r01_*): four lanes
 // read the 128 contiguous bytes (64 channels) of ONE sampled pixel per corner, each lane 32 bytes = one
 // deformable group when C/dg = 16, so the sampling geometry is computed once per 16 channels; offsets of the next
-// stage are prefetched while the current one is gathered; the fused fp16 pipeline blends with packed HFMA2.
+// stage are prefetched while the current one is gathered.
 //
 // Sampling semantics (bit-for-bit the reference's decisions, fp32 coordinate math):
 //   h_im = ho*stride - pad + i*dil + dh;  sample iff h_im > -1 && w_im > -1 && h_im < H && w_im < W
@@ -34,11 +34,8 @@ constexpr int DC_NPX = 1;                // output pixels per gather thread and 
 constexpr int DC_GATHER_THREADS = 512 / DC_NPX;
 constexpr int DC_THREADS = 192 + DC_GATHER_THREADS + 32;   // warps 0 B-producer, 1 MMA, 2-5 epilogue, 6.. gather, last: forwarder
 constexpr int DC_MAX_COUT = 512;
-constexpr int DC_REC_WORDS = 14;          // packed (pixel, group) record staged per gather thread: 18 offsets + 9 masks = 27 halfs
-constexpr int DC_SMEM_BYTES = DC_STAGES * (DC_A_BYTES + DC_B_BYTES) + DC_MAX_COUT * 4 + 256 + DC_REC_WORDS * DC_GATHER_THREADS * 4;
+constexpr int DC_SMEM_BYTES = DC_STAGES * (DC_A_BYTES + DC_B_BYTES) + DC_MAX_COUT * 4 + 256;
 constexpr int DC_TILE_H = 16, DC_TILE_W = 8;
-
-enum : int { OFF_NCHW_F32 = 0, OFF_PACK_F16 = 1 };
 
 struct DcnParams {
     const __half* x;          // NHWC fp16 [N][H][W][C] view
@@ -49,11 +46,8 @@ struct DcnParams {
     int kh, kw, stride, pad, dil;   // along H
     int stride_w, pad_w, dil_w;     // along W (DCNv1 passes independent pairs; v2 passes equal values)
     int dg, cpg;              // deformable groups, channels per group (multiple of 8)
-    int off_mode;
-    const float* offset;      // OFF_NCHW_F32: [N][dg*2*K][Ho][Wo]   (reference layout)
-    const float* mask;        //               [N][dg*K][Ho][Wo]; NULL = no modulation (DCNv1)
-    const __half* offpack;    // OFF_PACK_F16: [N][Ho][Wo][dg*32]: per group 18 offsets, 9 masks, 5 pad
-    int offpack_pix_stride;
+    const float* offset;      // [N][dg*2*K][Ho][Wo]   (reference layout)
+    const float* mask;        // [N][dg*K][Ho][Wo]; NULL = no modulation (DCNv1)
     const __half* wpack;      // [n_tile][chunk][tap][kc=8][BN][8] fp16
     int BN, n_tiles_n;
     EpiParams epi;            // epi.H/W == Ho/Wo
@@ -69,27 +63,6 @@ __device__ __align__(32) const uint32_t dcn_zero32[8] = {0, 0, 0, 0, 0, 0, 0, 0}
 
 struct DcnOff { float dh, dw, mk; };
 
-// 8 channels x 4 corners in packed fp16 (fused fp16 pipeline only; the fp32-layout operator keeps fp32 math)
-__device__ __forceinline__ uint4 dcn_blend8_h2(uint4 u0, uint4 u1, uint4 u2, uint4 u3, const float (&w)[4]) {
-    const __half2 w0 = __float2half2_rn(w[0]), w1 = __float2half2_rn(w[1]), w2 = __float2half2_rn(w[2]),
-                  w3 = __float2half2_rn(w[3]);
-    uint4 r;
-    uint32_t* ro = reinterpret_cast<uint32_t*>(&r);
-    const uint32_t* a = reinterpret_cast<const uint32_t*>(&u0);
-    const uint32_t* b = reinterpret_cast<const uint32_t*>(&u1);
-    const uint32_t* c = reinterpret_cast<const uint32_t*>(&u2);
-    const uint32_t* d = reinterpret_cast<const uint32_t*>(&u3);
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-        __half2 acc = __hmul2(w0, *reinterpret_cast<const __half2*>(&a[i]));
-        acc = __hfma2(w1, *reinterpret_cast<const __half2*>(&b[i]), acc);
-        acc = __hfma2(w2, *reinterpret_cast<const __half2*>(&c[i]), acc);
-        acc = __hfma2(w3, *reinterpret_cast<const __half2*>(&d[i]), acc);
-        ro[i] = *reinterpret_cast<uint32_t*>(&acc);
-    }
-    return r;
-}
-
 __device__ __forceinline__ void dcn_blend8(float (&acc)[8], uint4 u, float w) {
     const float2 a = unpack_h2(u.x), b = unpack_h2(u.y), c = unpack_h2(u.z), d = unpack_h2(u.w);
     acc[0] = fmaf(w, a.x, acc[0]); acc[1] = fmaf(w, a.y, acc[1]);
@@ -98,7 +71,6 @@ __device__ __forceinline__ void dcn_blend8(float (&acc)[8], uint4 u, float w) {
     acc[6] = fmaf(w, d.x, acc[6]); acc[7] = fmaf(w, d.y, acc[7]);
 }
 
-template <int OFFMODE, int EK>
 __global__ void __launch_bounds__(DC_THREADS, 1) dcn_fused_kernel(const DcnParams P) {
     extern __shared__ __align__(128) uint8_t smem[];
     uint8_t* a_smem = smem;
@@ -111,7 +83,6 @@ __global__ void __launch_bounds__(DC_THREADS, 1) dcn_fused_kernel(const DcnParam
     uint64_t* acc_full = bars + 3 * DC_STAGES;   // [2]
     uint64_t* acc_empty = acc_full + 2;          // [2]
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(acc_empty + 2);
-    uint32_t* rec_s = reinterpret_cast<uint32_t*>(reinterpret_cast<uint8_t*>(bars) + 256);   // [DC_REC_WORDS][DC_GATHER_THREADS]
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int tiles_x = (P.Wo + DC_TILE_W - 1) / DC_TILE_W;
@@ -199,7 +170,7 @@ __global__ void __launch_bounds__(DC_THREADS, 1) dcn_fused_kernel(const DcnParam
             for (int cc = 0; cc < P.BN; cc += 32) {
                 float v[32];
                 tmem_ld32(t0 + cc, v);
-                epi_store32<EK>(P.epi, has_bias ? bias_s : nullptr, v, img, y, x, nt * P.BN + cc, valid);
+                epi_store32<EK_NCHW>(P.epi, has_bias ? bias_s : nullptr, v, img, y, x, nt * P.BN + cc, valid);
             }
             tc_fence_before_sync();
             __syncwarp();
@@ -236,49 +207,17 @@ __global__ void __launch_bounds__(DC_THREADS, 1) dcn_fused_kernel(const DcnParam
         const long long plane = static_cast<long long>(Ho) * Wo;
         const float* const off_f = P.offset;
         const float* const msk_f = P.mask;
-        const __half* const off_h = P.offpack;
-        const long long ops = P.offpack_pix_stride;
         const bool wide = P.x_wide != 0;
 
-        // Packed-offset pipeline with one group per lane: the 64-byte (pixel, group) record is fetched ONCE per chunk with four
-        // 16-byte loads and parked in shared memory (word-major, so the per-tap reads are conflict-free 4-byte LDS).  Reading
-        // 4 + 2 bytes per tap straight from global memory cost as many L1 wavefronts as the whole corner gather (two loads per
-        // stage, 16 lines each: the lanes of a warp sit in 8 pixels x 4 groups, 64 bytes apart).
-        const bool staged = OFFMODE == OFF_PACK_F16 && cpg >= 16 && DC_NPX == 1;
-        const uint32_t rec_slot = smem_u32(rec_s) + (threadIdx.x - (DC_THREADS - 32 - DC_GATHER_THREADS)) * 4;
-        struct Pix { int m, hb, wb; bool ok; const __half* rec; const float* ob; const float* mb; };
-        auto stage_record = [&](const Pix& px, int g) {
-            uint4 r[4];
-#pragma unroll
-            for (int q = 0; q < 4; ++q) r[q] = px.ok ? ldg_nc_v4(px.rec + g * 32 + q * 8) : make_uint4(0, 0, 0, 0);
-            const uint32_t* w = reinterpret_cast<const uint32_t*>(r);
-#pragma unroll
-            for (int q = 0; q < DC_REC_WORDS; ++q) sts_u32(rec_slot + q * (DC_GATHER_THREADS * 4), w[q]);
-        };
+        struct Pix { int m, hb, wb; bool ok; const float* ob; const float* mb; };
         auto fetch = [&](const Pix& px, int g, int tap) -> DcnOff {
             DcnOff o;
             o.dh = o.dw = o.mk = 0.f;
-            if (staged) {
-                const uint32_t w0 = lds_u32(rec_slot + tap * (DC_GATHER_THREADS * 4));
-                const uint32_t wm = lds_u32(rec_slot + (9 + (tap >> 1)) * (DC_GATHER_THREADS * 4));
-                const float2 hw = unpack_h2(w0);
-                const float2 mm = unpack_h2(wm);
-                o.dh = hw.x; o.dw = hw.y; o.mk = (tap & 1) ? mm.y : mm.x;
-                return o;
-            }
             if (px.ok) {
-                if (OFFMODE == OFF_NCHW_F32) {
-                    const float* ob = px.ob + (static_cast<long long>(g) * 2 * K + 2 * tap) * plane;
-                    o.dh = __ldg(ob);
-                    o.dw = __ldg(ob + plane);
-                    o.mk = msk_f ? __ldg(px.mb + (static_cast<long long>(g) * K + tap) * plane) : 1.f;
-                } else {
-                    const __half* rec = px.rec + g * 32;
-                    const __half2 hw2 = *reinterpret_cast<const __half2*>(rec + 2 * tap);
-                    o.dh = __low2float(hw2);
-                    o.dw = __high2float(hw2);
-                    o.mk = __half2float(rec[18 + tap]);
-                }
+                const float* ob = px.ob + (static_cast<long long>(g) * 2 * K + 2 * tap) * plane;
+                o.dh = __ldg(ob);
+                o.dw = __ldg(ob + plane);
+                o.mk = msk_f ? __ldg(px.mb + (static_cast<long long>(g) * K + tap) * plane) : 1.f;
             }
             return o;
         };
@@ -319,13 +258,11 @@ __global__ void __launch_bounds__(DC_THREADS, 1) dcn_fused_kernel(const DcnParam
                 px[i].hb = ho * strd - pad;
                 px[i].wb = wo * strd_w - pad_w;
                 const long long pix = static_cast<long long>(ho) * Wo + wo;
-                px[i].rec = (OFFMODE == OFF_PACK_F16) ? off_h + (static_cast<long long>(img) * plane + pix) * ops : nullptr;
-                px[i].ob = (OFFMODE == OFF_NCHW_F32) ? off_f + static_cast<long long>(img) * dg * 2 * K * plane + pix : nullptr;
-                px[i].mb = (OFFMODE == OFF_NCHW_F32) ? msk_f + static_cast<long long>(img) * dg * K * plane + pix : nullptr;
+                px[i].ob = off_f + static_cast<long long>(img) * dg * 2 * K * plane + pix;
+                px[i].mb = msk_f + static_cast<long long>(img) * dg * K * plane + pix;
             }
             // software pipeline: the (dh, dw, mask) triples of the NEXT stage are fetched while this one is gathered
             int g0 = (kc0 * 8) / cpg, g1 = (kc0 * 8 + 8) / cpg;
-            if (staged) stage_record(px[0], g0);
             DcnOff nxt[DC_NPX][2];
 #pragma unroll
             for (int i = 0; i < DC_NPX; ++i) {
@@ -375,7 +312,6 @@ __global__ void __launch_bounds__(DC_THREADS, 1) dcn_fused_kernel(const DcnParam
                         const int t1 = last_tap ? 0 : tap + 1;
                         const int h0 = last_tap ? ng0 : g0, h1 = last_tap ? ng1 : g1;
                         if (!(last_tap && chunk + 1 == nchunks)) {
-                            if (staged && last_tap) stage_record(px[0], h0);     // this chunk's record is no longer needed
 #pragma unroll
                             for (int i = 0; i < DC_NPX; ++i) {
                                 nxt[i][0] = fetch(px[i], h0, t1);
@@ -391,18 +327,13 @@ __global__ void __launch_bounds__(DC_THREADS, 1) dcn_fused_kernel(const DcnParam
                     for (int i = 0; i < DC_NPX; ++i)
 #pragma unroll
                         for (int a = 0; a < 2; ++a) {
-                            uint4 r;
-                            if (OFFMODE == OFF_PACK_F16) {
-                                r = dcn_blend8_h2(u[i][a][0], u[i][a][1], u[i][a][2], u[i][a][3], cn[i][a].w);
-                            } else {
-                                float acc[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-                                dcn_blend8(acc, u[i][a][0], cn[i][a].w[0]);
-                                dcn_blend8(acc, u[i][a][1], cn[i][a].w[1]);
-                                dcn_blend8(acc, u[i][a][2], cn[i][a].w[2]);
-                                dcn_blend8(acc, u[i][a][3], cn[i][a].w[3]);
-                                r = make_uint4(pack_h2(acc[0], acc[1]), pack_h2(acc[2], acc[3]), pack_h2(acc[4], acc[5]),
-                                               pack_h2(acc[6], acc[7]));
-                            }
+                            float acc[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+                            dcn_blend8(acc, u[i][a][0], cn[i][a].w[0]);
+                            dcn_blend8(acc, u[i][a][1], cn[i][a].w[1]);
+                            dcn_blend8(acc, u[i][a][2], cn[i][a].w[2]);
+                            dcn_blend8(acc, u[i][a][3], cn[i][a].w[3]);
+                            const uint4 r = make_uint4(pack_h2(acc[0], acc[1]), pack_h2(acc[2], acc[3]), pack_h2(acc[4], acc[5]),
+                                                       pack_h2(acc[6], acc[7]));
                             sts_v4(dst + a * DC_A_LBO + px[i].m * 16, r);
                         }
                     __syncwarp();

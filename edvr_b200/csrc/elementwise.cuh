@@ -79,10 +79,9 @@ __global__ void nhwc_f16_to_nchw_f32_kernel(const __half* __restrict__ src, floa
 }
 
 // ------------------------------------------------------------------ weight packer
-// out element group (16 B): [nt][s1][s2][kc][n][0..7]; one thread per group.
-__global__ void pack_weight_kernel(const float* __restrict__ w, int cout, int cin, int ktaps,
-                                   const int* __restrict__ row_map, int BN, int n_tiles_n,
-                                   int tap_major, __half* __restrict__ out) {
+// out element group (16 B): [nt][chunk][tap][kc][n][0..7]; one thread per group.
+__global__ void pack_weight_kernel(const float* __restrict__ w, int cout, int cin, int ktaps, int BN, int n_tiles_n,
+                                   __half* __restrict__ out) {
     const int nchunks = cin / 64;
     const long long total = static_cast<long long>(n_tiles_n) * nchunks * ktaps * 8 * BN;
     for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < total;
@@ -90,12 +89,10 @@ __global__ void pack_weight_kernel(const float* __restrict__ w, int cout, int ci
         long long r = i;
         const int n = r % BN; r /= BN;
         const int kc = r % 8; r /= 8;
-        int tap, chunk;
-        if (tap_major) { chunk = r % nchunks; r /= nchunks; tap = r % ktaps; r /= ktaps; }
-        else           { tap = r % ktaps; r /= ktaps; chunk = r % nchunks; r /= nchunks; }
+        const int tap = r % ktaps; r /= ktaps;
+        const int chunk = r % nchunks; r /= nchunks;
         const int nt = static_cast<int>(r);
-        const int prow = nt * BN + n;
-        int srow = row_map ? row_map[prow] : prow;
+        int srow = nt * BN + n;
         if (srow >= cout) srow = -1;
         H8 v;
 #pragma unroll
@@ -113,8 +110,7 @@ __device__ __forceinline__ void bf8_store(__half* p, const H8& r) {
                                               pack_bf2(r.v[4], r.v[5]), pack_bf2(r.v[6], r.v[7]));
 }
 template <bool BF16>
-__global__ void pack_weight_pair_kernel(const float* __restrict__ w, int cout, int cin, int ktaps,
-                                        const int* __restrict__ row_map, int BN, int n_tiles_n,
+__global__ void pack_weight_pair_kernel(const float* __restrict__ w, int cout, int cin, int ktaps, int BN, int n_tiles_n,
                                         __half* __restrict__ out) {
     const int nchunks = cin / 32, half = BN / 2;
     const long long total = static_cast<long long>(n_tiles_n) * 2 * nchunks * ktaps * 4 * half;
@@ -128,8 +124,7 @@ __global__ void pack_weight_pair_kernel(const float* __restrict__ w, int cout, i
         const int chunk = r % nchunks; r /= nchunks;
         const int rank = r % 2; r /= 2;
         const int nt = static_cast<int>(r);
-        const int prow = nt * BN + rank * half + row;
-        int srow = row_map ? row_map[prow] : prow;
+        int srow = nt * BN + rank * half + row;
         if (srow >= cout) srow = -1;
         H8 v;
 #pragma unroll
@@ -237,13 +232,10 @@ __global__ void pack_weight_pair_dgrad_kernel(const float* __restrict__ w, int c
         if (BF16) bf8_store(out + i * 8, v); else h8_store(out + i * 8, v);
     }
 }
-__global__ void pack_bias_kernel(const float* __restrict__ b, int cout, const int* __restrict__ row_map,
-                                 int n_packed, float* __restrict__ out) {
+__global__ void pack_bias_kernel(const float* __restrict__ b, int cout, int n_packed, float* __restrict__ out) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n_packed) return;
-    int s = row_map ? row_map[i] : i;
-    if (s >= cout) s = -1;
-    out[i] = (b != nullptr && s >= 0) ? b[s] : 0.f;
+    out[i] = (b != nullptr && i < cout) ? b[i] : 0.f;
 }
 
 // ------------------------------------------------------------------ conv_first (Cin = 3)

@@ -12,7 +12,6 @@ enum : int { OUT_SAME = 0, OUT_PIXSHUF2 = 1, OUT_STRIDE2 = 2 };
 // (a single do-everything epilogue made the conv kernels 40-77 KB of SASS; profiles/r01_ncu_conv2_icache.txt).
 enum : int { EK_PLAIN = 0,    // fp16 NHWC out (+ optional fp16 residual)
              EK_F32 = 1,      // fp32 residual stream in/out (+ optional fp16 copy): trunk blocks
-             EK_PACK = 2,     // conv_offset: packed DCN record (sigmoid on mask logits, |offset| sum)
              EK_PIXSHUF = 3,  // PixelShuffle(2) store
              EK_STRIDE2 = 4,  // even-pixel store
              EK_NCHW = 5,     // fp32 NCHW out (reference operator layout)
@@ -34,7 +33,6 @@ struct EpiParams {
     float* out_nchw;          // [N][nchw_C][H][W] fp32 (reference op layout)
     int nchw_C;
     int out_mode;             // OUT_*
-    float* absmean_acc;       // ACT_DCN_PACK: sum |offset| accumulator (optional)
     int f32_blocked;          // res32 / out32 in the tile-blocked layout (blocked32_offset)
     int res16_wide;           // res16 view is 32-byte aligned per 16 channels: 2 x LDG.256 instead of 4 x LDG.128
     int bf16;                 // operands and the 16-bit output are bf16 (training step); CTA-pair kernel, plain TMA store only
@@ -49,8 +47,7 @@ __host__ __device__ __forceinline__ long long blocked32_block(int img, int y, in
     return (((tile * 2 + sub) * 4 + (m >> 5)) * (C >> 5) + chunk) * 1024 + (m & 31) * 4;
 }
 
-// v: 32 consecutive accumulator channels [c0, c0+32) of output pixel (img, y, x).
-// Every lane of the warp must call this (shuffles inside); `valid` masks the memory traffic.
+// v: 32 consecutive accumulator channels [c0, c0+32) of output pixel (img, y, x); `valid` masks the memory traffic.
 // EXT16: the caller stores the fp16 NHWC copy itself (TMA store in conv_pair.cuh); v[] holds the final values on return.
 // Residual prefetch for the blocked fp32 stream (trunk blocks): the eight float4 slots epi_store32 would read for channels
 // [c0, c0+32) of pixel (img, y, x), issued early so that their DRAM latency overlaps the wait for the accumulator and the
@@ -85,32 +82,13 @@ __device__ __forceinline__ void epi_prefetch_res16(const EpiParams& p, int img, 
 template <int EK = EK_GENERIC, bool EXT16 = false>
 __device__ __forceinline__ void epi_store32(const EpiParams& p, const float* __restrict__ bias_s,
                                             float (&v)[32], int img, int y, int x, int c0,
-                                            bool valid, float* abs_sum = nullptr, const float4* res_pre = nullptr) {
+                                            bool valid, const float4* res_pre = nullptr) {
     if (bias_s != nullptr) {
 #pragma unroll
         for (int j = 0; j < 32; ++j) v[j] += bias_s[c0 + j];
     }
     constexpr bool G = EK == EK_GENERIC;
-    if ((G || EK == EK_PACK) && p.act == ACT_DCN_PACK) {
-        // channel j of each 32-group: [0,18) offsets (dh,dw per tap), [18,27) mask logits, rest pad
-        float s = 0.f;
-#pragma unroll
-        for (int j = 0; j < 18; ++j) s += fabsf(v[j]);
-#pragma unroll
-        for (int j = 18; j < 27; ++j) v[j] = sigmoidf_fast(v[j]);
-        if (abs_sum != nullptr) {
-            // the caller keeps a per-lane running sum and does ONE reduction + atomic per warp at the end of the kernel: an
-            // atomic per 32x32 block meant 400K atomics on one address per conv_offset launch (~0.3 ms of a 0.9 ms kernel)
-            *abs_sum += valid ? s : 0.f;
-        } else if (p.absmean_acc != nullptr) {
-            s = valid ? s : 0.f;
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-            if (lane_id() == 0) atomicAdd(p.absmean_acc, s);
-        }
-    } else {
-        act_inplace<32>(v, p.act);
-    }
+    act_inplace<32>(v, p.act);
     if (!valid) return;
 
     const size_t pix = (static_cast<size_t>(img) * p.H + y) * p.W + x;
@@ -155,7 +133,7 @@ __device__ __forceinline__ void epi_store32(const EpiParams& p, const float* __r
         }
     }
 
-    if ((G && p.out_mode == OUT_SAME) || EK == EK_PLAIN || EK == EK_F32 || EK == EK_PACK || EK == EK_NCHW) {
+    if ((G && p.out_mode == OUT_SAME) || EK == EK_PLAIN || EK == EK_F32 || EK == EK_NCHW) {
         if (!EXT16 && EK != EK_NCHW && p.out16 != nullptr) {
             uint4* o = reinterpret_cast<uint4*>(p.out16 + pix * p.out16_pix_stride + p.out16_ch_off + c0);
 #pragma unroll
@@ -206,14 +184,6 @@ __device__ __forceinline__ void epi_store32(const EpiParams& p, const float* __r
             o[q] = make_uint4(pack_h2(v[q * 8 + 0], v[q * 8 + 1]), pack_h2(v[q * 8 + 2], v[q * 8 + 3]),
                               pack_h2(v[q * 8 + 4], v[q * 8 + 5]), pack_h2(v[q * 8 + 6], v[q * 8 + 7]));
     }
-}
-
-// end-of-kernel flush of the running |offset| sum kept by an epilogue warp (see epi_store32, abs_sum)
-__device__ __forceinline__ void epi_flush_abs_sum(const EpiParams& p, float s) {
-    if (p.absmean_acc == nullptr) return;
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-    if (lane_id() == 0) atomicAdd(p.absmean_acc, s);
 }
 
 }  // namespace eb

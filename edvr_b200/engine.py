@@ -18,7 +18,7 @@ but restructured for the hardware:
 import torch
 
 from . import ops
-from .ops import ACT_DCN_PACK, ACT_LRELU, ACT_NONE, ACT_RELU, OUT_PIXSHUF2, OUT_STRIDE2, View
+from .ops import ACT_LRELU, ACT_NONE, ACT_RELU, OUT_PIXSHUF2, OUT_STRIDE2, View
 
 
 class _Arena:

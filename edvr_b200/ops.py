@@ -9,8 +9,7 @@ import os
 import torch
 
 from . import _lib as L
-from ._lib import (ACT_DCN_PACK, ACT_LRELU, ACT_NONE, ACT_RELU, ACT_SIGMOID, OUT_PIXSHUF2,  # noqa: F401
-                   OUT_SAME, OUT_STRIDE2)
+from ._lib import ACT_LRELU, ACT_NONE, ACT_RELU, ACT_SIGMOID, OUT_PIXSHUF2, OUT_SAME, OUT_STRIDE2  # noqa: F401
 
 
 LAUNCHES = [0]      # number of libedvr_b200 kernel launches issued through this module (bench.py: gpu_launches)
@@ -82,17 +81,12 @@ def _choose_bn(cout_packed):
     raise ValueError(f"packed Cout {cout_packed} must be a multiple of 32")
 
 
-def pack_conv(weight, bias=None, row_map=None, tap_major=False, cout_packed=None):
-    """weight: fp32 [Cout, Cin, k, k] (CUDA). row_map: optional LongTensor packed-row -> source row (-1 = 0)."""
+def pack_conv(weight, bias=None, cout_packed=None):
+    """weight: fp32 [Cout, Cin, k, k] (CUDA)."""
     assert weight.is_cuda and weight.dtype == torch.float32
     weight = weight.contiguous()
     cout, cin, k, _ = weight.shape
-    if row_map is not None:
-        cout_packed = int(row_map.numel())
-        rm = row_map.to(device=weight.device, dtype=torch.int32).contiguous()
-    else:
-        cout_packed = cout_packed or ((cout + 31) // 32) * 32
-        rm = None
+    cout_packed = cout_packed or ((cout + 31) // 32) * 32
     p = PackedConv()
     p.BN = _choose_bn(cout_packed)
     p.n_tiles = cout_packed // p.BN
@@ -101,40 +95,20 @@ def pack_conv(weight, bias=None, row_map=None, tap_major=False, cout_packed=None
     nbytes = L.lib().eb_packed_weight_bytes(cin, k * k, p.BN, p.n_tiles)
     p.w = torch.empty(nbytes // 2, dtype=torch.float16, device=weight.device)
     with _Rec("pack_weight", 1):
-        L.check(L.lib().eb_pack_weight(L.ptr(weight), cout, cin, k * k, L.ptr(rm), p.BN, p.n_tiles,
-                                       1 if tap_major else 0, L.ptr(p.w), L.stream_ptr()), "eb_pack_weight")
+        L.check(L.lib().eb_pack_weight(L.ptr(weight), cout, cin, k * k, p.BN, p.n_tiles, L.ptr(p.w), L.stream_ptr()),
+                "eb_pack_weight")
     p.wpair = None
-    if not tap_major and L.lib().eb_conv2d_pair_supported(cin, k, p.BN, p.n_tiles):
+    if L.lib().eb_conv2d_pair_supported(cin, k, p.BN, p.n_tiles):
         # second packing for the CTA-pair kernel (weights resident in shared memory), see conv_pair.cuh
         p.wpair = torch.empty(nbytes // 2, dtype=torch.float16, device=weight.device)
         with _Rec("pack_weight", 1):
-            L.check(L.lib().eb_pack_weight_pair(L.ptr(weight), cout, cin, k * k, L.ptr(rm), p.BN, p.n_tiles,
+            L.check(L.lib().eb_pack_weight_pair(L.ptr(weight), cout, cin, k * k, p.BN, p.n_tiles,
                                                 L.ptr(p.wpair), L.stream_ptr()), "eb_pack_weight_pair")
     b = torch.zeros(cout_packed, dtype=torch.float32, device=weight.device)
     if bias is not None:
-        if rm is None:
-            b[:cout] = bias.float()
-        else:
-            sel = rm >= 0
-            b[sel] = bias.float()[rm[sel].long()]
+        b[:cout] = bias.float()
     p.b = b
     return p
-
-
-def dcn_offset_row_map(dg, k2=9):
-    """conv_offset rows -> packed [g][32] layout: (dh,dw) x k2, then k2 mask logits, then pad.
-
-    Source rows follow the reference: offsets g*2*k2 + j, masks dg*2*k2 + g*k2 + k
-    (arch_util.py:244-247, deform_conv_cuda_kernel.cu:600-613).
-    """
-    assert k2 == 9
-    rm = torch.full((dg * 32,), -1, dtype=torch.int32)
-    for g in range(dg):
-        for j in range(18):
-            rm[g * 32 + j] = g * 18 + j
-        for k in range(9):
-            rm[g * 32 + 18 + k] = dg * 18 + g * 9 + k
-    return rm
 
 
 def _src(v, div=1, mul=1, keep=0, add=0):
@@ -162,7 +136,7 @@ class Blocked32:
 
 
 def _epi(pc_bias, act, out16=None, out32=None, res16=None, res32=None, out_nchw=None, nchw_C=0,
-         out_mode=OUT_SAME, absmean=None, bf16=False):
+         out_mode=OUT_SAME, bf16=False):
     e = L.Epilogue()
     e.bf16 = 1 if bf16 else 0
     e.bias = None if pc_bias is None else pc_bias.data_ptr()
@@ -185,12 +159,11 @@ def _epi(pc_bias, act, out16=None, out32=None, res16=None, res32=None, out_nchw=
     if out_nchw is not None:
         e.out_nchw, e.nchw_C = out_nchw.data_ptr(), nchw_C
     e.out_mode = out_mode
-    e.absmean_acc = None if absmean is None else absmean.data_ptr()
     return e
 
 
 def conv2d(pc, srcs, out16=None, act=ACT_NONE, res16=None, res32=None, out32=None, out_mode=OUT_SAME,
-           absmean=None, src_maps=None, N=None, out_nchw=None, nchw_C=0):
+           src_maps=None, N=None, out_nchw=None, nchw_C=0):
     """srcs: list of 1-2 Views (channel-concatenated input). src_maps: per-source (div, mul, keep, add)."""
     v0 = srcs[0]
     N = v0.N if N is None else N
@@ -200,14 +173,13 @@ def conv2d(pc, srcs, out16=None, act=ACT_NONE, res16=None, res32=None, out32=Non
         arr[i] = _src(v, *m)
     assert sum(v.C for v in srcs) == pc.cin, (sum(v.C for v in srcs), pc.cin)
     bf16 = v0.t.dtype == torch.bfloat16
-    e = _epi(pc.b, act, out16, out32, res16, res32, out_nchw=out_nchw, nchw_C=nchw_C, out_mode=out_mode, absmean=absmean,
-             bf16=bf16)
+    e = _epi(pc.b, act, out16, out32, res16, res32, out_nchw=out_nchw, nchw_C=nchw_C, out_mode=out_mode, bf16=bf16)
     opix = N * v0.H * v0.W if out_mode != OUT_STRIDE2 else N * ((v0.H + 1) // 2) * ((v0.W + 1) // 2)
     detail = ""
     if PROFILE is not None:
         detail = (f"{pc.cin}->{pc.cout} {N}x{v0.H}x{v0.W} act{act} mode{out_mode}"
                   f"{' res16' if res16 is not None else ''}{' res32' if res32 is not None else ''}"
-                  f"{' out32' if out32 is not None else ''}{' pack' if absmean is not None else ''}")
+                  f"{' out32' if out32 is not None else ''}")
     with _Rec(f"conv_igemm_{pc.ksize}x{pc.ksize}", 1, 2.0 * opix * pc.cout * pc.cin_real * pc.ksize * pc.ksize, detail):
         if pc.wpair is not None and USE_PAIR and os.environ.get("EDVR_B200_CONV_PAIR", "1") != "0":
             L.check(L.lib().eb_conv2d_pair(arr, len(srcs), N, v0.H, v0.W, pc.ksize, L.ptr(pc.wpair), pc.BN, pc.n_tiles,
@@ -215,14 +187,6 @@ def conv2d(pc, srcs, out16=None, act=ACT_NONE, res16=None, res32=None, out32=Non
         else:
             L.check(L.lib().eb_conv2d(arr, len(srcs), N, v0.H, v0.W, pc.ksize, L.ptr(pc.w), pc.BN, pc.n_tiles,
                                       ctypes.byref(e), L.stream_ptr()), "eb_conv2d")
-
-
-def dcn_nhwc(pc, x, offpack, dg, out16=None, act=ACT_NONE, out_nchw=None, nchw_C=0):
-    e = _epi(pc.b, act, out16, out_nchw=out_nchw, nchw_C=nchw_C)
-    with _Rec("dcn_fused", 1, 2.0 * x.N * x.H * x.W * pc.cout * pc.cin * 9, f"{x.N}x{x.H}x{x.W} C{x.C}"):
-        L.check(L.lib().eb_dcn_nhwc(L.ptr(x.t), x.pix_stride, x.ch_off, x.N, x.H, x.W, x.C, dg, L.ptr(offpack.t),
-                                    offpack.pix_stride, L.ptr(pc.w), pc.BN, pc.n_tiles, ctypes.byref(e),
-                                    L.stream_ptr()), "eb_dcn_nhwc")
 
 
 class OffsetMonitor:
@@ -268,15 +232,19 @@ class DcnSite:
     mode "pair" (default): ONE launch of the CTA-pair kernel (dcn_pair.cuh): conv_offset runs on the tensor cores inside the
     DCN kernel, overlapped with the gather; offsets and masks stay in tensor memory.  mode "fused": the single-CTA form of
     the same fusion (dcn_site.cuh; odd dg, more than one output-channel tile).  mode "split": conv_offset as a separate convolution writing the reference's fp32 NCHW
-    offset/mask-logit tensor, then the same DCN kernel reading it (used when dg*27 > 224).  mode "legacy": the round-1
-    pipeline (fp16 offset record, dcn_fused.cuh), kept for A/B timing only - its fp16 offsets miss the 1e-3 bar at
-    multi-pixel offsets."""
+    offset/mask-logit tensor, then the same DCN kernel reading it (used when dg*27 > 224).  `mode` (default: the
+    EDVR_B200_DCN_SITE environment variable, else "pair") is where the selection starts; a site that the requested kernel
+    cannot serve moves on to the next mode of pair -> fused -> split."""
+
+    MODES = ("pair", "fused", "split")
 
     def __init__(self, wo, bo, w, b, dg, mode=None):
+        mode = mode or os.environ.get("EDVR_B200_DCN_SITE", "pair")
+        if mode not in self.MODES:
+            raise ValueError(f"DcnSite mode {mode!r}: expected one of {', '.join(self.MODES)}")
         self.dg = dg
         self.C = w.shape[1]
         self.main = pack_conv(w, b)
-        mode = mode or os.environ.get("EDVR_B200_DCN_SITE", "pair")
         if mode == "pair" and not (w.shape[2] == 3 and self.main.wpair is not None and
                                    L.lib().eb_dcn_pair_supported(self.C, dg, self.main.BN, self.main.n_tiles)):
             mode = "fused"
@@ -300,10 +268,8 @@ class DcnSite:
                 L.check(L.lib().eb_dcn_site_pack_offset_weight(L.ptr(wo.contiguous()), L.ptr(None if bo is None else bo.contiguous()),
                                                                self.C, dg, L.ptr(self.wo_pack), L.ptr(self.bo_cols),
                                                                L.stream_ptr()), "eb_dcn_site_pack_offset_weight")
-        elif mode == "split":
-            self.offset = pack_conv(wo, bo, cout_packed=((dg * 27 + 127) // 128) * 128)
         else:
-            self.offset = pack_conv(wo, bo, row_map=dcn_offset_row_map(dg))
+            self.offset = pack_conv(wo, bo, cout_packed=((dg * 27 + 127) // 128) * 128)
         self._rec = {}
 
     def _raw(self, N, H, W, device):
@@ -311,31 +277,21 @@ class DcnSite:
         t = self._rec.get(key)
         if t is None:
             self._rec.clear()           # one shape at a time: the offsets are the largest temporary of the graph
-            if self.mode == "split":
-                t = torch.empty(N, self.n_off, H, W, dtype=torch.float32, device=device)
-            else:
-                t = new_act(N, H, W, self.dg * 32, device)
+            t = torch.empty(N, self.n_off, H, W, dtype=torch.float32, device=device)
             self._rec[key] = t
         return t
 
     def arena_record(self, arena, feat):
         """Scratch for the offsets shared by all sites of an executor (engine._Arena); None when nothing is materialised."""
-        if self.mode in ("pair", "fused"):
+        if self.mode != "split":
             return None
-        if self.mode == "split":
-            return arena.f32("offraw", feat.N, self.n_off, feat.H, feat.W)
-        return arena.act("offpack", feat.N, feat.H, feat.W, self.dg * 32)
+        return arena.f32("offraw", feat.N, self.n_off, feat.H, feat.W)
 
     def __call__(self, x, feat, out16=None, act=ACT_NONE, absmean=None, record=None, out_nchw=None):
         """out16: NHWC fp16 View, or out_nchw: fp32 [N, Cout, H, W] (the reference operator's layout)."""
         N, H, W = feat.N, feat.H, feat.W
         pc = self.main
         flops = 2.0 * N * H * W * pc.cout * pc.cin * 9
-        if self.mode == "legacy":
-            offp = record if record is not None else self._raw(N, H, W, feat.t.device)
-            conv2d(self.offset, [feat], out16=offp, act=ACT_DCN_PACK, absmean=absmean)
-            dcn_nhwc(pc, x, offp, self.dg, out16=out16, act=act, out_nchw=out_nchw, nchw_C=pc.cout)
-            return
         e = _epi(pc.b, act, out16, out_nchw=out_nchw, nchw_C=pc.cout)
         am = None if absmean is None else absmean.data_ptr()
         if self.mode == "pair":

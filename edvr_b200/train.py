@@ -62,7 +62,7 @@ def _pack_pair(weight, bias, bf16, dgrad_k=0):
             L.check(L.lib().eb_pack_weight_pair_dgrad(L.ptr(weight), cout, cin, k * k, kch, pc.BN, pc.n_tiles, L.ptr(pc.wpair),
                                                       1 if bf16 else 0, L.stream_ptr()), "eb_pack_weight_pair_dgrad")
         else:
-            L.check(L.lib().eb_pack_weight_pair_ex(L.ptr(weight), cout, cin, k * k, None, pc.BN, pc.n_tiles, L.ptr(pc.wpair),
+            L.check(L.lib().eb_pack_weight_pair_ex(L.ptr(weight), cout, cin, k * k, pc.BN, pc.n_tiles, L.ptr(pc.wpair),
                                                    1 if bf16 else 0, L.stream_ptr()), "eb_pack_weight_pair_ex")
     if bias is not None and cp == rows and bias.dtype == torch.float32 and bias.is_contiguous():
         pc.b = bias.detach()

@@ -18,7 +18,7 @@
  *          same ownership (caller allocates outputs; grad_weight / grad_bias are accumulated
  *          into, the other grads overwritten), `ones` / `columns` scratch handles dropped in
  *          favour of one caller-owned workspace.
- *   eb_conv2d / eb_dcn_nhwc / eb_* elementwise
+ *   eb_conv2d / eb_dcn_site / eb_dcn_site_pair / eb_* elementwise
  *       == the cuDNN / ATen dispatches behind nn.Conv2d, nn.LeakyReLU, nn.Upsample, nn.*Pool2d,
  *          nn.PixelShuffle, torch.cat in archs/edvr_arch.py:76-117,161-214,250-269,358-420 and
  *          archs/arch_util.py:92-95,243-257, on NHWC fp16 tensors (fp32 accumulation).
@@ -36,8 +36,7 @@ extern "C" {
 #define EB_ACT_NONE 0
 #define EB_ACT_RELU 1
 #define EB_ACT_LRELU 2      /* negative slope 0.1 (edvr_arch.py:70) */
-#define EB_ACT_DCN_PACK 3   /* conv_offset epilogue: per 32-ch group, ch 18..26 -> sigmoid */
-#define EB_ACT_SIGMOID 4
+#define EB_ACT_SIGMOID 4    /* 3 is unassigned: rejected with -2 */
 /* output index maps */
 #define EB_OUT_SAME 0
 #define EB_OUT_PIXSHUF2 1   /* nn.PixelShuffle(2) fused into the store */
@@ -66,7 +65,6 @@ typedef struct {
     float* out_nchw;          /* optional NCHW fp32 output [N][nchw_C][H][W] */
     int nchw_C;
     int out_mode;
-    float* absmean_acc;       /* optional: sum |offset| (EB_ACT_DCN_PACK), for the >50 warning */
     int f32_blocked;          /* res32/out32 use the tile-blocked private layout of eb_f32_blocked_elems() */
     int bf16;                 /* 1: inputs, packed weights and out16 are bf16 instead of fp16 (training step; eb_conv2d_pair,
                                  plain NHWC output only) */
@@ -86,11 +84,9 @@ int eb_selftest_mma_rate(int cta_group, int M, int N, int layout, int a_lbo, int
                          int kstep_bytes, int reps, unsigned long long* cycles, int* n_ctas, void* stream);
 
 /* ---- weight packing (device side; fp32 OIHW -> fp16 MMA-ready stages) ------------------
- * layout [n_tile][s1][s2][kc=8][BN][8]; tap_major=1: s1=tap,s2=chunk (DCN); 0: s1=chunk,s2=tap.
- * row_map (device int32[BN*n_tiles_n], or NULL=identity) maps packed row -> source row (-1 = zero). */
+ * layout [n_tile][chunk][tap][kc=8][BN][8]; packed rows >= cout are zero. */
 size_t eb_packed_weight_bytes(int cin, int ktaps, int BN, int n_tiles_n);
-int eb_pack_weight(const float* w_oihw, int cout, int cin, int ktaps, const int* row_map, int BN,
-                   int n_tiles_n, int tap_major, void* wpack, void* stream);
+int eb_pack_weight(const float* w_oihw, int cout, int cin, int ktaps, int BN, int n_tiles_n, void* wpack, void* stream);
 
 /* ---- dense convolution, NHWC fp16, 3x3 (pad 1) or 1x1, stride 1 (stride 2 via out_mode) ---- */
 int eb_conv2d(const eb_src_t* srcs, int nsrc, int N, int H, int W, int ksize, const void* wpack,
@@ -104,10 +100,9 @@ int eb_conv2d_stats(const eb_src_t* srcs, int nsrc, int N, int H, int W, int ksi
  * Cin * 9 * BN <= 147456, e.g. 128 -> 128; 2 = weights stream with the activation stages: 3x3 256 -> 128, every 1x1).  `wpair` is produced by
  * eb_pack_weight_pair (same size as eb_packed_weight_bytes); sources, epilogue and results as eb_conv2d. */
 int eb_conv2d_pair_supported(int cin, int ksize, int BN, int n_tiles_n);
-int eb_pack_weight_pair(const float* w, int cout, int cin, int ktaps, const int* row_map, int BN, int n_tiles_n,
-                        void* wpair, void* stream);
-int eb_pack_weight_pair_ex(const float* w, int cout, int cin, int ktaps, const int* row_map, int BN, int n_tiles_n,
-                           void* wpair, int bf16, void* stream);
+int eb_pack_weight_pair(const float* w, int cout, int cin, int ktaps, int BN, int n_tiles_n, void* wpair, void* stream);
+int eb_pack_weight_pair_ex(const float* w, int cout, int cin, int ktaps, int BN, int n_tiles_n, void* wpair, int bf16,
+                           void* stream);
 /* Weights of the DATA-GRADIENT convolution packed straight from the forward weights w[cout][cin][k][k]: row ci, K index co,
  * tap flipped (training step; k_channels = cout rounded up to a multiple of 64 = channels of the padded grad_out view). */
 int eb_pack_weight_pair_dgrad(const float* w, int cout, int cin, int ktaps, int k_channels, int BN, int n_tiles_n, void* wpair,
@@ -120,11 +115,6 @@ int eb_conv2d_pair(const eb_src_t* srcs, int nsrc, int N, int H, int W, int ksiz
  * epilogue owns them (16x16 tiles -> two 16x8 halves -> four 32-pixel quarters -> 32-channel chunks), so that every
  * warp-level float4 access is 512 contiguous bytes.  Returns the number of floats to allocate for [N,H,W,C]. */
 size_t eb_f32_blocked_elems(int N, int H, int W, int C);
-
-/* ---- DCNv2 forward on NHWC fp16 input with packed fp16 offsets/mask (fused pipeline) ---- */
-int eb_dcn_nhwc(const void* x, int x_pix_stride, int x_ch_off, int N, int H, int W, int C, int dg,
-                const void* offpack, int offpack_pix_stride, const void* wpack, int BN, int n_tiles_n,
-                const eb_epilogue_t* epi, void* stream);
 
 /* ---- Training step (BASELINE cfg 5): weight gradient of a dense 3x3 (pad 1, stride 1) or 1x1 convolution,
  *   grad_weight[co][ci][ky][kx] += scale * sum_{n,y,x} gy[n,y,x,co] * x[n, y+ky-1, x+kx-1, ci]

@@ -1,5 +1,6 @@
 """CPU tests of the host side: the C-ABI library loads and exports every declared symbol (no compute calls
-without a GPU), host-side packing maps, and the N>1 sharding logic on gloo with world_size 2."""
+without a GPU), argument validation that runs before any CUDA call, and the N>1 sharding logic on gloo with world_size 2."""
+import ctypes
 import json
 import os
 import re
@@ -37,15 +38,23 @@ def test_host_validation_without_gpu():
     assert b"workspace" in h.eb_last_error()
     assert h.eb_mdcn_forward_workspace(1, 64, 8, 8, 64, 3, 3) >= 8 * 8 * 64 * 2
     assert h.eb_packed_weight_bytes(128, 9, 128, 1) == 128 * 128 * 9 * 2
+    # activation code 3 is unassigned: the epilogue check rejects it before the kernel choice touches the device
+    src = (L.Src * 1)(L.Src(p.value, 64, 64, 0, 1, 1, 0, 0))
+    e = L.Epilogue(act=3, out16=p.value, out16_pix_stride=64)
+    assert h.eb_conv2d(src, 1, 1, 8, 8, 3, p, 128, 1, ctypes.byref(e), None) == -2
+    assert h.eb_conv2d_pair(src, 1, 1, 8, 8, 3, p, 128, 1, ctypes.byref(e), None) == -2
+    assert b"act 3" in h.eb_last_error()
 
 
-def test_dcn_offset_row_map():
-    from edvr_b200.ops import dcn_offset_row_map
-    rm = dcn_offset_row_map(8)
-    assert rm.numel() == 256
-    used = rm[rm >= 0]
-    assert sorted(used.tolist()) == list(range(216))          # every conv_offset row lands exactly once
-    assert rm[32 + 18].item() == 144 + 9 and rm[32].item() == 18 and rm[27].item() == -1
+def test_dcn_site_rejects_unknown_mode(monkeypatch):
+    """A mode outside pair / fused / split is an error, raised before any packing or CUDA call (CPU tensors here)."""
+    from edvr_b200.ops import DcnSite
+    wo, w = torch.zeros(8 * 27, 64, 3, 3), torch.zeros(64, 64, 3, 3)
+    with pytest.raises(ValueError, match="'legacy'"):
+        DcnSite(wo, None, w, None, 8, mode="legacy")
+    monkeypatch.setenv("EDVR_B200_DCN_SITE", "legacy")
+    with pytest.raises(ValueError, match="'legacy'"):
+        DcnSite(wo, None, w, None, 8)
 
 
 def test_missing_library_fails_loudly(monkeypatch):

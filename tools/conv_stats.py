@@ -1,4 +1,4 @@
-"""Role-level cycle counters of conv_igemm2 (eb_conv2d_stats) + isolated timing of one conv / one DCN call."""
+"""Role-level cycle counters of conv_igemm2 (eb_conv2d_stats) + isolated timing of one conv call."""
 import ctypes
 import os
 import sys
@@ -57,22 +57,6 @@ def conv_case(N, H, W, cin, cout, k, res32=False, label=""):
               f"epi: tmem {m[11]/tiles:.0f} p1 {m[12]/tiles:.0f} bar {m[13]/tiles:.0f} p2 {m[14]/tiles:.0f}", flush=True)
 
 
-def dcn_case(N, H, W, C, dg=8):
-    x = ops.nchw_to_nhwc(torch.randn(N, C, H, W, device="cuda"))
-    feat = ops.nchw_to_nhwc(torch.randn(N, C, H, W, device="cuda"))
-    wo = torch.randn(dg * 27, C, 3, 3, device="cuda") * 0.02
-    bo = torch.randn(dg * 27, device="cuda") * 0.5
-    w = torch.randn(C, C, 3, 3, device="cuda") / (C * 9) ** 0.5
-    po = ops.pack_conv(wo, bo, row_map=ops.dcn_offset_row_map(dg))
-    pw = ops.pack_conv(w, torch.zeros(C, device="cuda"))
-    offp = ops.new_act(N, H, W, dg * 32)
-    ops.conv2d(po, [feat], out16=offp, act=ops.ACT_DCN_PACK)
-    out = ops.new_act(N, H, W, C)
-    ms = time_it(lambda: ops.dcn_nhwc(pw, x, offp, dg, out16=out))
-    byts = N * H * W * (C * 2 + dg * 64 + C * 2) + C * C * 9 * 2
-    print(f"dcn N={N} {H}x{W} C={C}: {ms*1e3:.1f} us  {2.0*N*H*W*C*C*9/ms/1e9:.0f} TFLOP/s  {byts/ms/1e6:.0f} GB/s (fp16 algorithmic bytes)", flush=True)
-
-
 if __name__ == "__main__":
     conv_case(4, 180, 320, 128, 128, 3, label="trunk conv1")
     conv_case(4, 180, 320, 128, 128, 3, res32=True, label="trunk conv2")
@@ -82,6 +66,3 @@ if __name__ == "__main__":
     conv_case(4, 180, 320, 896, 256, 1, label="tsa fuse 1x1")
     conv_case(4, 720, 1280, 64, 64, 3, label="conv_hr")
     conv_case(4, 360, 640, 128, 256, 3, label="upconv2")
-    dcn_case(28, 180, 320, 128)
-    dcn_case(28, 90, 160, 128)
-    dcn_case(4, 180, 320, 128)

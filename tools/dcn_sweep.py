@@ -1,5 +1,5 @@
 """DCN site (conv_offset -> DCN) at several offset magnitudes: parity vs the C oracle on a small shape and device time
-of the two launches at full size.  `sigma` is the standard deviation of the sampling offsets in pixels (iid per pixel,
+of the site's launches at full size.  `sigma` is the standard deviation of the sampling offsets in pixels (iid per pixel,
 group and tap: the worst case for locality; trained EDVR offsets are smoother).
 
     python tools/dcn_sweep.py [--n 28] [--sigmas 0.02,3,10] [--json gpurun_out/dcn_sweep.json]
@@ -79,7 +79,7 @@ def main():
     ap.add_argument("--n", default="28,4")
     ap.add_argument("--sigmas", default="0.02,3,10")
     ap.add_argument("--json", default=os.path.join(ROOT, "gpurun_out", "dcn_sweep.json"))
-    ap.add_argument("--modes", default="pair,fused,legacy", help="ops.DcnSite modes to compare")
+    ap.add_argument("--modes", default="pair,fused", help="ops.DcnSite modes to compare")
     a = ap.parse_args()
     res = {"parity": [], "timing": []}
     for mode in a.modes.split(","):

@@ -51,13 +51,12 @@ def sec_conv():
     res = {}
     torch.manual_seed(1)
 
-    def run(name, N, H, W, cins, cout, k, act=ops.ACT_NONE, res16=False, out_mode=ops.OUT_SAME, maps=None,
-            row_map=None):
+    def run(name, N, H, W, cins, cout, k, act=ops.ACT_NONE, res16=False, out_mode=ops.OUT_SAME, maps=None):
         xs = [torch.randn(N if (maps is None or maps[i] is None) else maps[i][4], c, H, W, device="cuda")
               for i, c in enumerate(cins)]
         w = torch.randn(cout, sum(cins), k, k, device="cuda") * (1.0 / (sum(cins) * k * k) ** 0.5)
         b = torch.randn(cout, device="cuda") * 0.1
-        pc = ops.pack_conv(w, b, row_map=row_map)
+        pc = ops.pack_conv(w, b)
         views = [ops.nchw_to_nhwc(x) for x in xs]
         # reference on the fp16-rounded operands, fp32 math
         xr = []

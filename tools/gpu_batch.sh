@@ -7,7 +7,7 @@ if [[ "$stages" == *T* ]]; then
   timeout 1200 python -m pytest tests -m gpu -q 2>&1 | tail -40 > gpurun_out/${tag}_pytest_gpu.log; tail -4 gpurun_out/${tag}_pytest_gpu.log
 fi
 if [[ "$stages" == *S* ]]; then
-  timeout 400 python tools/dcn_sweep.py --modes pair,fused,legacy --n 28 --sigmas 0.02,3,10 --json gpurun_out/${tag}_dcn_sweep.json 2>&1 | grep timing | cut -c1-220
+  timeout 400 python tools/dcn_sweep.py --n 28 --sigmas 0.02,3,10 2>&1 | grep timing | cut -c1-220      # modes pair,fused; dcn_sweep.json
 fi
 if [[ "$stages" == *P* ]]; then
   timeout 200 python tools/dp_prof.py 28 0.02 0,127 2>&1 | cut -c1-400 | tee gpurun_out/${tag}_dcn_pair_role_timing.txt

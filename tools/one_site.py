@@ -1,5 +1,5 @@
 """Launch one DCN site (ops.DcnSite) a few times on one shape: ncu target.
-    python tools/one_site.py N H W C dg sigma [iters]      (mode: EDVR_B200_DCN_SITE=fused|split|legacy)"""
+    python tools/one_site.py N H W C dg sigma [iters]      (mode: EDVR_B200_DCN_SITE=pair|fused|split)"""
 import os
 import sys
 
