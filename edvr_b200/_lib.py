@@ -75,6 +75,15 @@ _SIGS = {
     "eb_dcn1_backward_workspace": (c_size_t, [c_int] * 13),
     "eb_dcn1_backward_input": (c_int, [c_void_p] * 6 + [c_int] * 15 + [c_void_p, c_size_t, c_void_p]),
     "eb_dcn1_backward_parameters": (c_int, [c_void_p] * 4 + [c_float] + [c_int] * 15 + [c_void_p, c_size_t, c_void_p]),
+    "eb_mdcn_forward_f64": (c_int, [c_void_p] * 6 + [c_int] * 12 + [c_void_p]),
+    "eb_mdcn_backward_f64_workspace": (c_size_t, [c_int] * 10),
+    "eb_mdcn_backward_f64": (c_int, [c_void_p] * 10 + [c_int] * 12 + [c_void_p, c_size_t, c_void_p]),
+    "eb_dcn1_forward_f64": (c_int, [c_void_p] * 4 + [c_int] * 15 + [c_void_p]),
+    "eb_dcn1_backward_input_f64_workspace": (c_size_t, [c_int] * 13),
+    "eb_dcn1_backward_parameters_f64_workspace": (c_size_t, [c_int] * 13),
+    "eb_dcn1_backward_input_f64": (c_int, [c_void_p] * 6 + [c_int] * 15 + [c_void_p, c_size_t, c_void_p]),
+    "eb_dcn1_backward_parameters_f64": (c_int, [c_void_p] * 4 + [ctypes.c_double] + [c_int] * 15 +
+                                        [c_void_p, c_size_t, c_void_p]),
     "eb_nchw_f32_to_nhwc_f16": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p]),
     "eb_nhwc_f16_to_nchw_f32": (c_int, [c_void_p, c_int, c_int, c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
     "eb_conv_first": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p]),

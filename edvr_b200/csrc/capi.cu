@@ -13,6 +13,7 @@
 #include "conv_pair.cuh"
 #include "conv_train.cuh"
 #include "dcn_backward.cuh"
+#include "dcn_f64.cuh"
 #include "dcn_fused.cuh"
 #include "dcn_site.cuh"
 #include "dcn_pair.cuh"
@@ -119,7 +120,7 @@ int set_smem(KernelT k, int bytes) {
 
 extern "C" {
 
-int eb_version(void) { return 101; }
+int eb_version(void) { return 102; }
 const char* eb_last_error(void) { return g_err; }
 
 int eb_selftest_umma(const void* A, const void* B, float* D, int N, int K, int variant, void* stream) {
@@ -1167,6 +1168,193 @@ int eb_dcn1_backward_parameters(const float* x, const float* offset, const float
                                 int pad_w, int dil_h, int dil_w, int groups, int dg, void* workspace, size_t workspace_bytes,
                                 void* stream) {
     return dcn_backward_impl("dcn1_backward_parameters", x, offset, nullptr, nullptr, grad_out, nullptr, nullptr, nullptr,
+                             grad_weight, nullptr, scale, false, true, N, C, H, W, Cout, kh, kw,
+                             Geo2{stride_h, stride_w, pad_h, pad_w, dil_h, dil_w}, groups, dg, workspace, workspace_bytes, stream);
+}
+
+// ---- fp64 reference-layout operator (dcn_f64.cuh) ---------------------------------------------------------------------
+namespace {
+constexpr int F64_MAX_Z = 65535;                                   // gridDim.z: images per launch
+constexpr size_t F64_GCOL_BYTES = static_cast<size_t>(256) << 20;  // gcol staging target (at least one image)
+
+// Argument checks shared by the fp64 entries: the statuses of the fp32 twins, without their C % 64 and Cout limits.
+int f64_check(const char* who, bool ptrs_ok, int N, int C, int H, int W, int Cout, int kh, int kw, Geo2 g, int groups, int dg,
+              F64Geom* G) {
+    if (!ptrs_ok) return fail(EB_ERR_NULLPTR, "%s: null pointer", who);
+    if (N < 0 || C < 1 || H < 1 || W < 1 || Cout < 1 || kh < 1 || kw < 1 || g.sh < 1 || g.sw < 1 || g.ph < 0 || g.pw < 0 ||
+        g.dh < 1 || g.dw < 1 || groups < 1 || dg < 1 || C % dg || C % groups || Cout % groups)
+        return fail(EB_ERR_INVALID_SHAPE, "%s: invalid shape", who);
+    if (groups != 1) return fail(EB_ERR_UNSUPPORTED, "%s: groups=%d (only 1; compose weight groups above the ABI)", who, groups);
+    const int Ho = (H + 2 * g.ph - (g.dh * (kh - 1) + 1)) / g.sh + 1;
+    const int Wo = (W + 2 * g.pw - (g.dw * (kw - 1) + 1)) / g.sw + 1;
+    if (Ho < 1 || Wo < 1) return fail(EB_ERR_INVALID_SHAPE, "%s: empty output", who);
+    if (static_cast<long long>(N) * Ho * Wo > 0x7fffffffLL || static_cast<long long>(C) * kh * kw > 0x7fffffffLL)
+        return fail(EB_ERR_UNSUPPORTED, "%s: more than 2^31 output pixels or C*kh*kw", who);
+    // the GEMM grids put C*kh*kw (gcol, wgrad) and Cout (forward) tiles on gridDim.y
+    if ((static_cast<long long>(C) * kh * kw + F64_BN - 1) / F64_BN > F64_MAX_Z || (Cout + F64_BN - 1) / F64_BN > F64_MAX_Z)
+        return fail(EB_ERR_UNSUPPORTED, "%s: C*kh*kw or Cout above %d", who, F64_MAX_Z * F64_BN);
+    *G = F64Geom{N, C, H, W, Cout, kh, kw, g.sh, g.sw, g.ph, g.pw, g.dh, g.dw, dg, Ho, Wo};
+    return EB_OK;
+}
+
+int f64_forward_impl(const char* who, const double* x, const double* offset, const double* mask, const double* weight,
+                     const double* bias, double* out, int N, int C, int H, int W, int Cout, int kh, int kw, Geo2 g, int groups,
+                     int dg, void* stream, bool need_mask) {
+    if (N == 0 && C > 0 && H > 0 && W > 0 && Cout > 0) return EB_OK;
+    F64Geom G;
+    if (int rc = f64_check(who, x && offset && (mask || !need_mask) && weight && out, N, C, H, W, Cout, kh, kw, g, groups, dg, &G))
+        return rc;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    F64FwdOp op;
+    op.G = G; op.x = x; op.offset = offset; op.mask = mask; op.weight = weight; op.bias = bias; op.out = out;
+    op.M = G.Ho * G.Wo; op.N = Cout;
+    for (int n0 = 0; n0 < N; n0 += F64_MAX_Z) {
+        op.n_first = n0;
+        const dim3 grid((op.M + F64_BM - 1) / F64_BM, (Cout + F64_BN - 1) / F64_BN, N - n0 < F64_MAX_Z ? N - n0 : F64_MAX_Z);
+        f64_gemm_kernel<F64FwdOp><<<grid, F64_THREADS, 0, st>>>(op);
+    }
+    return check_launch(who);
+}
+
+struct F64BwdWs {
+    size_t per_image;           // gcol bytes of one image
+    size_t gcol, part;          // bytes of the input side (gcol of `chunk` images) and of the grad_weight partials
+    int chunk;                  // images per gcol pass at the minimum workspace
+    int q_per_split, splits;    // grad_weight split-K over the N*Ho*Wo pixels (shapes only: reproducible everywhere)
+    // workspace of a call computing the input side, the parameter side or both (they reuse it one after the other)
+    size_t need(bool want_input, bool want_param) const {
+        const size_t a = want_input ? gcol : 0, b = want_param ? part : 0;
+        return up256(a > b ? a : b);
+    }
+};
+F64BwdWs f64_bwd_ws(int N, int C, int Cout, int K, int HWo) {
+    F64BwdWs w;
+    w.per_image = static_cast<size_t>(C) * K * HWo * 8;
+    size_t chunk = F64_GCOL_BYTES / w.per_image;
+    if (chunk > static_cast<size_t>(N)) chunk = N;
+    if (chunk > static_cast<size_t>(F64_MAX_Z)) chunk = F64_MAX_Z;
+    w.chunk = chunk < 1 ? 1 : static_cast<int>(chunk);
+    const long long Q = static_cast<long long>(N) * HWo;
+    long long qps = (Q + 31) / 32;
+    if (qps < 2048) qps = 2048;
+    w.q_per_split = static_cast<int>((qps + F64_BK - 1) / F64_BK * F64_BK);
+    w.splits = static_cast<int>((Q + w.q_per_split - 1) / w.q_per_split);
+    w.gcol = w.chunk * w.per_image;
+    w.part = static_cast<size_t>(w.splits) * Cout * C * K * 8;
+    return w;
+}
+
+size_t f64_bwd_workspace(int N, int C, int H, int W, int Cout, int kh, int kw, Geo2 g, bool want_input, bool want_param) {
+    if (N < 1 || C < 1 || H < 1 || W < 1 || Cout < 1 || kh < 1 || kw < 1 || g.sh < 1 || g.sw < 1 || g.dh < 1 || g.dw < 1)
+        return 256;
+    const int Ho = (H + 2 * g.ph - (g.dh * (kh - 1) + 1)) / g.sh + 1;
+    const int Wo = (W + 2 * g.pw - (g.dw * (kw - 1) + 1)) / g.sw + 1;
+    if (Ho < 1 || Wo < 1) return 256;
+    return f64_bwd_ws(N, C, Cout, kh * kw, Ho * Wo).need(want_input, want_param);
+}
+
+// `want_input` -> grad_x, grad_offset (and grad_mask when mask != NULL), overwritten; `want_param` ->
+// grad_weight += scale * dW, grad_bias += db.  The two sides share the workspace one after the other.
+int f64_backward_impl(const char* who, const double* x, const double* offset, const double* mask, const double* weight,
+                      const double* grad_out, double* grad_x, double* grad_offset, double* grad_mask, double* grad_weight,
+                      double* grad_bias, double scale, bool want_input, bool want_param, int N, int C, int H, int W, int Cout,
+                      int kh, int kw, Geo2 g, int groups, int dg, void* workspace, size_t workspace_bytes, void* stream) {
+    if (N == 0 && C > 0 && H > 0 && W > 0 && Cout > 0) return EB_OK;
+    const bool ptrs_ok = x && offset && grad_out && (!want_input || (weight && grad_x && grad_offset)) &&
+                         (!want_param || grad_weight);
+    F64Geom G;
+    if (int rc = f64_check(who, ptrs_ok, N, C, H, W, Cout, kh, kw, g, groups, dg, &G)) return rc;
+    const int K = kh * kw, HWo = G.Ho * G.Wo, CK = C * K;
+    const F64BwdWs ws = f64_bwd_ws(N, C, Cout, K, HWo);
+    const size_t need = ws.need(want_input, want_param);
+    if (!workspace || workspace_bytes < need)
+        return fail(EB_ERR_WORKSPACE, "%s: workspace %zu < %zu", who, workspace_bytes, need);
+    if (!al16(workspace)) return fail(EB_ERR_ALIGNMENT, "%s: workspace must be 16-byte aligned", who);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    double* buf = static_cast<double*>(workspace);
+    if (want_input) {
+        cudaMemsetAsync(grad_x, 0, static_cast<size_t>(N) * C * H * W * 8, st);
+        size_t fit = workspace_bytes / ws.per_image;             // a larger workspace takes more images per pass
+        int chunk = fit > static_cast<size_t>(N) ? N : static_cast<int>(fit);
+        if (chunk > F64_MAX_Z) chunk = F64_MAX_Z;
+        if (chunk < ws.chunk) chunk = ws.chunk;
+        F64GcolOp op;
+        op.G = G; op.weight = weight; op.grad_out = grad_out; op.gcol = buf; op.M = HWo; op.N = CK;
+        for (int n0 = 0; n0 < N; n0 += chunk) {
+            const int nc = N - n0 < chunk ? N - n0 : chunk;
+            op.n_first = n0;
+            f64_gemm_kernel<F64GcolOp><<<dim3((HWo + F64_BM - 1) / F64_BM, (CK + F64_BN - 1) / F64_BN, nc), F64_THREADS, 0, st>>>(op);
+            f64_coord_scatter_kernel<<<grid_1d(static_cast<long long>(nc) * dg * K * HWo, 256), 256, 0, st>>>(
+                G, x, offset, mask, buf, n0, nc, grad_x, grad_offset, mask ? grad_mask : nullptr);
+        }
+        if (int rc = check_launch(who)) return rc;
+    }
+    if (want_param) {
+        F64WgradOp op;
+        op.G = G; op.x = x; op.offset = offset; op.mask = mask; op.grad_out = grad_out; op.part = buf;
+        op.M = Cout; op.N = CK; op.q_per_split = ws.q_per_split; op.Q = N * HWo;
+        f64_gemm_kernel<F64WgradOp><<<dim3((Cout + F64_BM - 1) / F64_BM, (CK + F64_BN - 1) / F64_BN, ws.splits), F64_THREADS, 0, st>>>(op);
+        const long long n = static_cast<long long>(Cout) * CK;
+        f64_wgrad_reduce_kernel<<<grid_1d(n, 256), 256, 0, st>>>(buf, ws.splits, n, scale, grad_weight);
+        if (grad_bias) f64_bias_kernel<<<Cout, 256, 0, st>>>(grad_out, grad_bias, N, Cout, HWo);
+        if (int rc = check_launch(who)) return rc;
+    }
+    return EB_OK;
+}
+}  // namespace
+
+int eb_mdcn_forward_f64(const double* x, const double* offset, const double* mask, const double* weight, const double* bias,
+                        double* out, int N, int C, int H, int W, int Cout, int kh, int kw, int stride, int pad, int dil,
+                        int groups, int dg, void* stream) {
+    return f64_forward_impl("mdcn_forward_f64", x, offset, mask, weight, bias, out, N, C, H, W, Cout, kh, kw,
+                            Geo2{stride, stride, pad, pad, dil, dil}, groups, dg, stream, true);
+}
+
+int eb_dcn1_forward_f64(const double* x, const double* offset, const double* weight, double* out, int N, int C, int H, int W,
+                        int Cout, int kh, int kw, int stride_h, int stride_w, int pad_h, int pad_w, int dil_h, int dil_w,
+                        int groups, int dg, void* stream) {
+    return f64_forward_impl("dcn1_forward_f64", x, offset, nullptr, weight, nullptr, out, N, C, H, W, Cout, kh, kw,
+                            Geo2{stride_h, stride_w, pad_h, pad_w, dil_h, dil_w}, groups, dg, stream, false);
+}
+
+size_t eb_mdcn_backward_f64_workspace(int N, int C, int H, int W, int Cout, int kh, int kw, int stride, int pad, int dil) {
+    return f64_bwd_workspace(N, C, H, W, Cout, kh, kw, Geo2{stride, stride, pad, pad, dil, dil}, true, true);
+}
+
+size_t eb_dcn1_backward_input_f64_workspace(int N, int C, int H, int W, int Cout, int kh, int kw, int stride_h, int stride_w,
+                                            int pad_h, int pad_w, int dil_h, int dil_w) {
+    return f64_bwd_workspace(N, C, H, W, Cout, kh, kw, Geo2{stride_h, stride_w, pad_h, pad_w, dil_h, dil_w}, true, false);
+}
+
+size_t eb_dcn1_backward_parameters_f64_workspace(int N, int C, int H, int W, int Cout, int kh, int kw, int stride_h,
+                                                 int stride_w, int pad_h, int pad_w, int dil_h, int dil_w) {
+    return f64_bwd_workspace(N, C, H, W, Cout, kh, kw, Geo2{stride_h, stride_w, pad_h, pad_w, dil_h, dil_w}, false, true);
+}
+
+int eb_mdcn_backward_f64(const double* x, const double* offset, const double* mask, const double* weight,
+                         const double* grad_out, double* grad_x, double* grad_offset, double* grad_mask, double* grad_weight,
+                         double* grad_bias, int N, int C, int H, int W, int Cout, int kh, int kw, int stride, int pad, int dil,
+                         int groups, int dg, void* workspace, size_t workspace_bytes, void* stream) {
+    if (!(N == 0) && (!mask || !grad_mask)) return fail(EB_ERR_NULLPTR, "mdcn_backward_f64: null pointer");
+    return f64_backward_impl("mdcn_backward_f64", x, offset, mask, weight, grad_out, grad_x, grad_offset, grad_mask,
+                             grad_weight, grad_bias, 1.0, true, true, N, C, H, W, Cout, kh, kw,
+                             Geo2{stride, stride, pad, pad, dil, dil}, groups, dg, workspace, workspace_bytes, stream);
+}
+
+int eb_dcn1_backward_input_f64(const double* x, const double* offset, const double* weight, const double* grad_out,
+                               double* grad_x, double* grad_offset, int N, int C, int H, int W, int Cout, int kh, int kw,
+                               int stride_h, int stride_w, int pad_h, int pad_w, int dil_h, int dil_w, int groups, int dg,
+                               void* workspace, size_t workspace_bytes, void* stream) {
+    return f64_backward_impl("dcn1_backward_input_f64", x, offset, nullptr, weight, grad_out, grad_x, grad_offset, nullptr,
+                             nullptr, nullptr, 1.0, true, false, N, C, H, W, Cout, kh, kw,
+                             Geo2{stride_h, stride_w, pad_h, pad_w, dil_h, dil_w}, groups, dg, workspace, workspace_bytes, stream);
+}
+
+int eb_dcn1_backward_parameters_f64(const double* x, const double* offset, const double* grad_out, double* grad_weight,
+                                    double scale, int N, int C, int H, int W, int Cout, int kh, int kw, int stride_h,
+                                    int stride_w, int pad_h, int pad_w, int dil_h, int dil_w, int groups, int dg,
+                                    void* workspace, size_t workspace_bytes, void* stream) {
+    return f64_backward_impl("dcn1_backward_parameters_f64", x, offset, nullptr, nullptr, grad_out, nullptr, nullptr, nullptr,
                              grad_weight, nullptr, scale, false, true, N, C, H, W, Cout, kh, kw,
                              Geo2{stride_h, stride_w, pad_h, pad_w, dil_h, dil_w}, groups, dg, workspace, workspace_bytes, stream);
 }

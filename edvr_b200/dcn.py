@@ -36,6 +36,15 @@ def _f32c(t):
     return t.detach().to(torch.float32).contiguous()
 
 
+def _all_f64(*ts):
+    """True when every given tensor (None = absent) is float64: such calls run the double-precision kernels."""
+    return all(t is None or t.dtype == torch.float64 for t in ts)
+
+
+def _f64c(t):
+    return t.detach().contiguous()
+
+
 class ModulatedDeformConvFunction(Function):
 
     @staticmethod
@@ -48,6 +57,11 @@ class ModulatedDeformConvFunction(Function):
             raise NotImplementedError
         if weight.requires_grad or mask.requires_grad or offset.requires_grad or input.requires_grad:
             ctx.save_for_backward(input, offset, mask, weight, bias if ctx.with_bias else input.new_empty(1))
+        ctx.f64 = _all_f64(input, offset, mask, weight, bias)
+        if ctx.f64:
+            return ops.mdcn_forward(_f64c(input), _f64c(offset), _f64c(mask), _f64c(weight),
+                                    _f64c(bias) if ctx.with_bias else None, stride, padding, dilation, groups,
+                                    deformable_groups)
         out = ops.mdcn_forward(_f32c(input), _f32c(offset), _f32c(mask), _f32c(weight),
                                _f32c(bias) if ctx.with_bias else None, stride, padding, dilation, groups,
                                deformable_groups)
@@ -59,6 +73,11 @@ class ModulatedDeformConvFunction(Function):
         if not grad_output.is_cuda:
             raise NotImplementedError
         input, offset, mask, weight, bias = ctx.saved_tensors
+        if ctx.f64:
+            gx, goff, gmask, gw, gb = _mdcn_backward_raw(_f64c(input), _f64c(offset), _f64c(mask), _f64c(weight),
+                                                         _f64c(grad_output.double()), ctx.with_bias, ctx.stride,
+                                                         ctx.padding, ctx.dilation, ctx.groups, ctx.deformable_groups)
+            return gx, goff, gmask, gw, gb, None, None, None, None, None
         gx, goff, gmask, gw, gb = mdcn_backward(_f32c(input), _f32c(offset), _f32c(mask), _f32c(weight),
                                                 _f32c(grad_output), ctx.with_bias, ctx.stride, ctx.padding,
                                                 ctx.dilation, ctx.groups, ctx.deformable_groups)
@@ -90,7 +109,7 @@ def _mdcn_backward_raw(x, offset, mask, weight, grad_out, with_bias, stride, pad
     if groups > 1:          # composed from per-group calls (see ops.group_slices); shared deformable groups accumulate
         gx, gw = torch.empty_like(x), torch.empty_like(weight)
         goff, gmask = torch.zeros_like(offset), torch.zeros_like(mask)
-        gb = torch.zeros(Cout, dtype=torch.float32, device=x.device) if with_bias else None
+        gb = torch.zeros(Cout, dtype=x.dtype, device=x.device) if with_bias else None
         for gi in range(groups):
             cs, os_, fs, ms, dgg = ops.group_slices(C, Cout, kh * kw, groups, dg, gi)
             r = _mdcn_backward_raw(x[:, cs].contiguous(), offset[:, fs].contiguous(), mask[:, ms].contiguous(),
@@ -106,7 +125,15 @@ def _mdcn_backward_raw(x, offset, mask, weight, grad_out, with_bias, stride, pad
     goff = torch.empty_like(offset)
     gmask = torch.empty_like(mask)
     gw = torch.zeros_like(weight)
-    gb = torch.zeros(Cout, dtype=torch.float32, device=x.device) if with_bias else None
+    gb = torch.zeros(Cout, dtype=x.dtype, device=x.device) if with_bias else None
+    if x.dtype == torch.float64:        # every tensor fp64: the double-precision kernels, no scaling needed
+        need = L.lib().eb_mdcn_backward_f64_workspace(N, C, H, W, Cout, kh, kw, stride, padding, dilation)
+        ws = torch.empty(max(need, 16), dtype=torch.uint8, device=x.device)
+        L.check(L.lib().eb_mdcn_backward_f64(L.ptr(x), L.ptr(offset), L.ptr(mask), L.ptr(weight), L.ptr(grad_out),
+                                             L.ptr(gx), L.ptr(goff), L.ptr(gmask), L.ptr(gw), L.ptr(gb), N, C, H, W, Cout,
+                                             kh, kw, stride, padding, dilation, groups, dg, L.ptr(ws), ws.numel(),
+                                             L.stream_ptr()), "eb_mdcn_backward_f64")
+        return gx, goff, gmask, gw, gb
     need = L.lib().eb_mdcn_backward_workspace(N, C, H, W, Cout, kh, kw, stride, padding, dilation)
     ws = torch.empty(max(need, 16), dtype=torch.uint8, device=x.device)
     L.check(L.lib().eb_mdcn_backward(L.ptr(x), L.ptr(offset), L.ptr(mask), L.ptr(weight), L.ptr(grad_out),
@@ -135,9 +162,11 @@ class DeformConvFunction(Function):
             raise NotImplementedError
         step = min(ctx.im2col_step, input.shape[0])
         assert (input.shape[0] % step) == 0, "im2col step must divide batchsize"
-        output = torch.empty(out_shape, dtype=torch.float32, device=input.device)
+        ctx.f64 = _all_f64(input, offset, weight)
+        cv = _f64c if ctx.f64 else _f32c
+        output = torch.empty(out_shape, dtype=torch.float64 if ctx.f64 else torch.float32, device=input.device)
         from . import deform_conv_ext as ext
-        ext.deform_conv_forward(_f32c(input), _f32c(weight), _f32c(offset), output, None, None, weight.size(3),
+        ext.deform_conv_forward(cv(input), cv(weight), cv(offset), output, None, None, weight.size(3),
                                 weight.size(2), ctx.stride[1], ctx.stride[0], ctx.padding[1], ctx.padding[0],
                                 ctx.dilation[1], ctx.dilation[0], ctx.groups, ctx.deformable_groups, step)
         return output.to(input.dtype)
@@ -154,13 +183,14 @@ class DeformConvFunction(Function):
         from . import deform_conv_ext as ext
         geom = (weight.size(3), weight.size(2), ctx.stride[1], ctx.stride[0], ctx.padding[1], ctx.padding[0],
                 ctx.dilation[1], ctx.dilation[0], ctx.groups, ctx.deformable_groups)
-        x, off, go = _f32c(input), _f32c(offset), _f32c(grad_output)
+        cv = (lambda t: _f64c(t.double())) if ctx.f64 else _f32c       # fp64 calls keep fp64 (grad_output included)
+        x, off, go = cv(input), cv(offset), cv(grad_output)
         if ctx.needs_input_grad[0] or ctx.needs_input_grad[1]:
             gx, goff = torch.empty_like(x), torch.empty_like(off)
-            ext.deform_conv_backward_input(x, off, go, gx, goff, _f32c(weight), None, *geom, step)
+            ext.deform_conv_backward_input(x, off, go, gx, goff, cv(weight), None, *geom, step)
             grad_input, grad_offset = gx.to(input.dtype), goff.to(offset.dtype)
         if ctx.needs_input_grad[2]:
-            gw = torch.zeros(weight.shape, dtype=torch.float32, device=weight.device)
+            gw = torch.zeros(weight.shape, dtype=x.dtype, device=weight.device)
             ext.deform_conv_backward_parameters(x, off, go, gw, None, None, *geom, 1, step)
             grad_weight = gw.to(weight.dtype)
         return grad_input, grad_offset, grad_weight, None, None, None, None, None, None
@@ -240,6 +270,7 @@ class ModulatedDeformConvPack(ModulatedDeformConv):
     def _fusable(self, x):
         k = self.kernel_size
         return (not torch.is_grad_enabled() and x.is_cuda and k == (3, 3) and self.stride == 1 and self.padding == 1
+                and not (x.dtype == torch.float64 and self.weight.dtype == torch.float64)   # fp64 module: fp64 operator
                 and self.dilation == 1 and self.groups == 1 and self.in_channels % 64 == 0
                 and ((self.in_channels // self.deformable_groups) == 8 or (self.in_channels // self.deformable_groups) % 16 == 0))
 

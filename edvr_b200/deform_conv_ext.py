@@ -25,6 +25,12 @@ def _f32(t):
     return t if (t.dtype == torch.float32 and t.is_contiguous()) else t.float().contiguous()
 
 
+def _all_f64(*ts):
+    """True when every floating tensor of a call (None = absent) is float64: such calls run the double-precision entry
+    points as given - no cast and no grad_out scaling."""
+    return all(t is None or t.dtype == torch.float64 for t in ts)
+
+
 def _pow2_scale(grad_out):
     """Power of two s (computed on the device, no host sync) with amax(|grad_out|) * s in [2^9, 2^10): the backward kernels
     carry grad_out and W^T grad_out as fp16 tensor-core operands, so gradients of a mean-reduced loss (~1e-6 per pixel)
@@ -62,6 +68,13 @@ def modulated_deform_conv_forward(input, weight, bias, ones, offset, mask, outpu
                                                 kernel_w, stride_h, pad_h, dilation_h, group, deformable_group, L.ptr(ws),
                                                 ws.numel(), L.stream_ptr()), "eb_mdcn_forward_f16")
         return
+    if _all_f64(input, weight, offset, mask, output, bias if with_bias else None):
+        from . import ops          # groups > 1: the per-group composition of ops.mdcn_forward, each call fp64
+        with torch.cuda.device(input.device):
+            output.copy_(ops.mdcn_forward(input, offset.contiguous(), mask.contiguous(), weight,
+                                          bias.contiguous() if with_bias else None, stride_h, pad_h, dilation_h, group,
+                                          deformable_group))
+        return
     x, w, off, m = _f32(input), _f32(weight), _f32(offset), _f32(mask)
     b = _f32(bias) if with_bias else None
     if group > 1:           # deform_conv_cuda.cpp:536-568: one GEMM per weight group; composed from per-group calls
@@ -93,6 +106,20 @@ def modulated_deform_conv_backward(input, weight, bias, ones, offset, mask, colu
         raise RuntimeError("edvr_b200: anisotropic stride/pad/dilation is not supported")
     N, C, H, W = input.shape
     Cout = weight.shape[0]
+    if _all_f64(input, weight, offset, mask, grad_input, grad_weight, grad_offset, grad_mask, grad_output,
+                *((bias, grad_bias) if with_bias else ())):
+        from .dcn import _mdcn_backward_raw       # groups > 1: its per-group composition, each call fp64
+        with torch.cuda.device(input.device):
+            gx, goff, gm, gw, gb = _mdcn_backward_raw(input, offset.contiguous(), mask.contiguous(), weight,
+                                                      grad_output.contiguous(), bool(with_bias), stride_h, pad_h,
+                                                      dilation_h, group, deformable_group)
+        grad_input.copy_(gx)
+        grad_offset.copy_(goff)
+        grad_mask.copy_(gm)
+        grad_weight.add_(gw)
+        if with_bias:
+            grad_bias.add_(gb)
+        return
     x, w, off, m = _f32(input), _f32(weight), _f32(offset), _f32(mask)
     sc = _pow2_scale(grad_output)
     go = (grad_output.float() * sc).contiguous()
@@ -193,7 +220,8 @@ def deform_conv_forward(input, weight, offset, output, columns, ones, kW, kH, dW
     if N % im2col_step:
         raise RuntimeError("im2col step must divide batchsize")                  # deform_conv_cuda.cpp:189
     Cout = weight.shape[0]
-    x, w, off = _f32(input4), _f32(weight), _f32(offset4)
+    f64 = _all_f64(input4, weight, offset4, output)
+    x, w, off = (input4.contiguous(), weight, offset4.contiguous()) if f64 else (_f32(input4), _f32(weight), _f32(offset4))
     shape = (N, Cout, Ho, Wo) if input.dim() == 4 else (Cout, Ho, Wo)
     if tuple(output.shape) != shape:
         output.resize_(shape)
@@ -202,11 +230,20 @@ def deform_conv_forward(input, weight, offset, output, columns, ones, kW, kH, dW
         parts = []
         for gi in range(group):
             cs, os_, fs, _ms, dgg = group_slices(C, Cout, kH * kW, group, deformable_group, gi)
-            part = torch.empty(N, Cout // group, Ho, Wo, dtype=torch.float32, device=input.device)
+            part = torch.empty(N, Cout // group, Ho, Wo, dtype=x.dtype, device=input.device)
             deform_conv_forward(x[:, cs].contiguous(), w[os_].contiguous(), off[:, fs].contiguous(), part, columns, ones, kW, kH,
                                 dW, dH, padW, padH, dilationW, dilationH, 1, dgg, im2col_step)
             parts.append(part)
         output.copy_(torch.cat(parts, 1).reshape(shape))
+        return 1
+    if f64:
+        out64 = output if output.is_contiguous() else torch.empty(output.shape, dtype=torch.float64, device=output.device)
+        with torch.cuda.device(input.device):
+            L.check(L.lib().eb_dcn1_forward_f64(L.ptr(x), L.ptr(off), L.ptr(w), L.ptr(out64), N, C, H, W, Cout, kH, kW, dH,
+                                                dW, padH, padW, dilationH, dilationW, group, deformable_group,
+                                                L.stream_ptr()), "eb_dcn1_forward_f64")
+        if out64 is not output:
+            output.copy_(out64)
         return 1
     out32, copy_back = _out_buf(output)
     need = L.lib().eb_mdcn_forward_workspace(N, C, H, W, Cout, kH, kW)
@@ -231,12 +268,13 @@ def deform_conv_backward_input(input, offset, gradOutput, gradInput, gradOffset,
     if N % im2col_step:
         raise RuntimeError("im2col step must divide batchsize")
     Cout = weight.shape[0]
-    x, w, off = _f32(input4), _f32(weight), _f32(offset4)
+    f64 = _all_f64(input4, offset4, go4, gradInput, gradOffset, weight)
+    x, w, off = (input4.contiguous(), weight, offset4.contiguous()) if f64 else (_f32(input4), _f32(weight), _f32(offset4))
     if group > 1:           # composed from per-group calls; deformable groups shared between weight groups accumulate
         from .ops import group_slices
-        gx4 = torch.empty(input4.shape, dtype=torch.float32, device=input.device)
-        goff4 = torch.zeros(offset4.shape, dtype=torch.float32, device=input.device)
-        go4f = go4.float()
+        gx4 = torch.empty(input4.shape, dtype=x.dtype, device=input.device)
+        goff4 = torch.zeros(offset4.shape, dtype=x.dtype, device=input.device)
+        go4f = go4.to(x.dtype)
         for gi in range(group):
             cs, os_, fs, _ms, dgg = group_slices(C, Cout, kH * kW, group, deformable_group, gi)
             xg, og = x[:, cs].contiguous(), off[:, fs].contiguous()
@@ -247,6 +285,18 @@ def deform_conv_backward_input(input, offset, gradOutput, gradInput, gradOffset,
             goff4[:, fs] += gog
         gradInput.copy_(gx4.reshape(gradInput.shape))
         gradOffset.copy_(goff4.reshape(gradOffset.shape))
+        return 1
+    if f64:
+        gx, goff = torch.empty(input4.shape, dtype=torch.float64, device=input.device), torch.empty_like(off)
+        need = L.lib().eb_dcn1_backward_input_f64_workspace(N, C, H, W, Cout, kH, kW, dH, dW, padH, padW, dilationH, dilationW)
+        ws = torch.empty(max(need, 16), dtype=torch.uint8, device=input.device)
+        with torch.cuda.device(input.device):
+            L.check(L.lib().eb_dcn1_backward_input_f64(L.ptr(x), L.ptr(off), L.ptr(w), L.ptr(go4.contiguous()), L.ptr(gx),
+                                                       L.ptr(goff), N, C, H, W, Cout, kH, kW, dH, dW, padH, padW, dilationH,
+                                                       dilationW, group, deformable_group, L.ptr(ws), ws.numel(),
+                                                       L.stream_ptr()), "eb_dcn1_backward_input_f64")
+        gradInput.copy_(gx.reshape(gradInput.shape))
+        gradOffset.copy_(goff.reshape(gradOffset.shape))
         return 1
     sc = _pow2_scale(go4)
     go = (go4.float() * sc).contiguous()
@@ -275,17 +325,30 @@ def deform_conv_backward_parameters(input, offset, gradOutput, gradWeight, colum
     if N % im2col_step:
         raise RuntimeError("im2col step must divide batchsize")
     Cout = gradWeight.shape[0]
-    x, off = _f32(input4), _f32(offset4)
+    f64 = _all_f64(input4, offset4, go4, gradWeight)
+    x, off = (input4.contiguous(), offset4.contiguous()) if f64 else (_f32(input4), _f32(offset4))
     if group > 1:           # deform_conv_cuda.cpp:455-470 per weight group; composed from per-group calls
         from .ops import group_slices
-        go4f = go4.float()
+        go4f = go4.to(x.dtype)
         for gi in range(group):
             cs, os_, fs, _ms, dgg = group_slices(C, Cout, kH * kW, group, deformable_group, gi)
-            gwg = torch.zeros(gradWeight[os_].shape, dtype=torch.float32, device=gradWeight.device)
+            gwg = torch.zeros(gradWeight[os_].shape, dtype=x.dtype, device=gradWeight.device)
             deform_conv_backward_parameters(x[:, cs].contiguous(), off[:, fs].contiguous(), go4f[:, os_].contiguous(), gwg,
                                             columns, ones, kW, kH, dW, dH, padW, padH, dilationW, dilationH, 1, dgg, scale,
                                             im2col_step)
             gradWeight[os_] += gwg.to(gradWeight.dtype)
+        return 1
+    if f64:
+        gw = torch.zeros(gradWeight.shape, dtype=torch.float64, device=gradWeight.device)
+        need = L.lib().eb_dcn1_backward_parameters_f64_workspace(N, C, H, W, Cout, kH, kW, dH, dW, padH, padW, dilationH,
+                                                                 dilationW)
+        ws = torch.empty(max(need, 16), dtype=torch.uint8, device=input.device)
+        with torch.cuda.device(input.device):
+            L.check(L.lib().eb_dcn1_backward_parameters_f64(L.ptr(x), L.ptr(off), L.ptr(go4.contiguous()), L.ptr(gw),
+                                                            float(scale), N, C, H, W, Cout, kH, kW, dH, dW, padH, padW,
+                                                            dilationH, dilationW, group, deformable_group, L.ptr(ws),
+                                                            ws.numel(), L.stream_ptr()), "eb_dcn1_backward_parameters_f64")
+        gradWeight.add_(gw)
         return 1
     sc = _pow2_scale(go4)
     go = (go4.float() * sc).contiguous()

@@ -405,8 +405,9 @@ def group_slices(C, Cout, K, groups, dg, gi):
 
 
 def mdcn_forward(x, offset, mask, weight, bias, stride, padding, dilation, groups, dg, workspace=None):
-    """Reference-layout operator (fp32 NCHW) through eb_mdcn_forward.  Weight groups > 1 (deform_conv_cuda.cpp:536-568) are
-    composed from per-group calls on channel slices - EDVR itself always uses groups == 1."""
+    """Reference-layout operator (fp32 NCHW) through eb_mdcn_forward, or through eb_mdcn_forward_f64 when x is float64
+    (then every tensor is float64 and contiguous).  Weight groups > 1 (deform_conv_cuda.cpp:536-568) are composed from
+    per-group calls on channel slices - EDVR itself always uses groups == 1."""
     N, C, H, W = x.shape
     Cout, _, kh, kw = weight.shape
     if groups > 1:
@@ -419,6 +420,13 @@ def mdcn_forward(x, offset, mask, weight, bias, stride, padding, dilation, group
         return torch.cat(outs, 1)
     Ho = (H + 2 * padding - (dilation * (kh - 1) + 1)) // stride + 1
     Wo = (W + 2 * padding - (dilation * (kw - 1) + 1)) // stride + 1
+    if x.dtype == torch.float64:
+        out = torch.empty(N, Cout, Ho, Wo, dtype=torch.float64, device=x.device)
+        with _Rec("mdcn_forward_f64", 1):
+            L.check(L.lib().eb_mdcn_forward_f64(L.ptr(x), L.ptr(offset), L.ptr(mask), L.ptr(weight), L.ptr(bias),
+                                                L.ptr(out), N, C, H, W, Cout, kh, kw, stride, padding, dilation, groups,
+                                                dg, L.stream_ptr()), "eb_mdcn_forward_f64")
+        return out
     out = torch.empty(N, Cout, Ho, Wo, dtype=torch.float32, device=x.device)
     need = L.lib().eb_mdcn_forward_workspace(N, C, H, W, Cout, kh, kw)
     if workspace is None or workspace.numel() < need:

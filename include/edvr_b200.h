@@ -170,7 +170,7 @@ int eb_mdcn_forward(const float* x, const float* offset, const float* mask, cons
                     void* workspace, size_t workspace_bytes, void* stream);
 /* Half-precision entry (the reference dispatches its kernels on at::Half too: deform_conv_cuda_kernel.cu:781): every tensor
  * fp16 in the reference layouts.  fp16 tensor-core operands (the input as given), fp32 offsets / masks / accumulation, one
- * rounding of the result to fp16.  fp64 tensors have no entry point: callers convert (the B1 shim does). */
+ * rounding of the result to fp16.  fp64 tensors have their own entry points (the _f64 functions below). */
 size_t eb_mdcn_forward_f16_workspace(int N, int C, int H, int W, int Cout, int kh, int kw, int dg);
 int eb_mdcn_forward_f16(const void* x, const void* offset, const void* mask, const void* weight, const void* bias /* or NULL */,
                         void* out, int N, int C, int H, int W, int Cout, int kh, int kw, int stride, int pad, int dil,
@@ -201,6 +201,40 @@ int eb_dcn1_backward_parameters(const float* x, const float* offset, const float
                                 int N, int C, int H, int W, int Cout, int kh, int kw, int stride_h, int stride_w, int pad_h,
                                 int pad_w, int dil_h, int dil_w, int groups, int dg, void* workspace, size_t workspace_bytes,
                                 void* stream);
+
+/* ---- Double-precision operator (csrc/dcn_f64.cuh): the reference also dispatches on double (deform_conv_cuda_kernel.cu:781,
+ * 813,846).  Same layouts, ownership and statuses as the fp32 entries above with double in place of float, and every number
+ * stays fp64 (coordinates, bilinear weights, masks, products, accumulators; the GEMMs run on fp64 mma.sync).  Any kh x kw,
+ * C, Cout and dg with C % dg == 0 (no C % 64 or Cout limit); groups == 1 (-2 otherwise, as above).  The forwards need no
+ * workspace.  The backwards take one of at least the bytes their eb_*_f64_workspace() function returns: the column gradient
+ * of a chunk of images for the input side (at least one image; a larger workspace takes more per pass), the split-K
+ * partials of grad_weight for the parameter side, the larger of the two for eb_mdcn_backward_f64.  Shapes whose
+ * C*kh*kw or Cout exceed 65535 * 64 answer -2.  grad_offset,
+ * grad_mask, grad_weight and grad_bias are bit-reproducible; grad_x is an fp64 atomic scatter. */
+int eb_mdcn_forward_f64(const double* x, const double* offset, const double* mask, const double* weight,
+                        const double* bias /* NULL = no bias */, double* out, int N, int C, int H, int W, int Cout, int kh,
+                        int kw, int stride, int pad, int dil, int groups, int dg, void* stream);
+size_t eb_mdcn_backward_f64_workspace(int N, int C, int H, int W, int Cout, int kh, int kw, int stride, int pad, int dil);
+int eb_mdcn_backward_f64(const double* x, const double* offset, const double* mask, const double* weight,
+                         const double* grad_out, double* grad_x, double* grad_offset, double* grad_mask, double* grad_weight,
+                         double* grad_bias /* NULL = no bias */, int N, int C, int H, int W, int Cout, int kh, int kw,
+                         int stride, int pad, int dil, int groups, int dg, void* workspace, size_t workspace_bytes,
+                         void* stream);
+int eb_dcn1_forward_f64(const double* x, const double* offset, const double* weight, double* out, int N, int C, int H, int W,
+                        int Cout, int kh, int kw, int stride_h, int stride_w, int pad_h, int pad_w, int dil_h, int dil_w,
+                        int groups, int dg, void* stream);
+size_t eb_dcn1_backward_input_f64_workspace(int N, int C, int H, int W, int Cout, int kh, int kw, int stride_h, int stride_w,
+                                            int pad_h, int pad_w, int dil_h, int dil_w);
+size_t eb_dcn1_backward_parameters_f64_workspace(int N, int C, int H, int W, int Cout, int kh, int kw, int stride_h,
+                                                 int stride_w, int pad_h, int pad_w, int dil_h, int dil_w);
+int eb_dcn1_backward_input_f64(const double* x, const double* offset, const double* weight, const double* grad_out,
+                               double* grad_x, double* grad_offset, int N, int C, int H, int W, int Cout, int kh, int kw,
+                               int stride_h, int stride_w, int pad_h, int pad_w, int dil_h, int dil_w, int groups, int dg,
+                               void* workspace, size_t workspace_bytes, void* stream);
+int eb_dcn1_backward_parameters_f64(const double* x, const double* offset, const double* grad_out, double* grad_weight,
+                                    double scale, int N, int C, int H, int W, int Cout, int kh, int kw, int stride_h,
+                                    int stride_w, int pad_h, int pad_w, int dil_h, int dil_w, int groups, int dg,
+                                    void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- layout / elementwise stages of the EDVR graph (all NHWC fp16 unless noted) --------- */
 int eb_nchw_f32_to_nhwc_f16(const float* src, void* dst, int N, int C, int H, int W,
